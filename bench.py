@@ -4,6 +4,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched under torchrun by the driver)
     python bench.py --impl reference ...                     (the reference's CPU path on the host cores)
+    python bench.py ... --dump-outputs DIR                   (also write what the timed steps computed, DIR/*.npy)
 
 One JSON line on stdout (rank 0).  A "step" is one full KGEModel.train_step: gather+score+loss+backward, dense
 Adam, loss read-back excluded for `value` (inputs resident in HBM) and included for `e2e` (host batches).
@@ -177,6 +178,34 @@ def peaks():
             p = json.load(f)
             return p, "measured (MEASURED_PEAKS.json)"
     return {"hbm_gbs": 6650.0, "bf16_tflops_sustained": 1418.0}, "fallback (B200_PROFILING.md)"
+
+
+def row_sample(table, budget, seed=0):
+    """Rows of a (rows, dim) device table as float32 host data, at most `budget` bytes: every row when they fit, else a
+    fixed seeded sample of rows in ascending order (the same rows on every run of the same workload)."""
+    t = table.detach().reshape(table.shape[0], -1)
+    k = min(t.shape[0], max(1, budget // (t.shape[1] * 4)))
+    if k < t.shape[0]:
+        rows = np.sort(np.random.RandomState(seed).choice(t.shape[0], k, replace=False))
+        t = t[rows]
+    return t.float().cpu().numpy()
+
+
+def train_outputs(m, loss_buffer):
+    """What a caller of the timed train step receives from its last call: the loss buffer's [positive_sample_loss,
+    negative_sample_loss, loss, regularization] and every trainable table (each at most 28 MB: a seeded row sample)."""
+    out = {"train_losses": loss_buffer[:4].cpu().numpy()}
+    for name, p in m.named_parameters():
+        if p.requires_grad:
+            out[name] = row_sample(p, 28 << 20)
+    return out
+
+
+def dump_outputs(path, arrays):
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        np.save(os.path.join(path, name + ".npy"), a if a.dtype in (np.float32, np.float64) else a.astype(np.float64))
 
 
 def host_cores():
@@ -386,8 +415,9 @@ class Bench:
                                       uni_weight=False, regularization=reg)
         return m, opt, targs, st
 
-    def train(self, wl, steps, warmup, e2e=True):
-        """value (device-resident inputs), kernel timing, e2e (public KGEModel.train_step on pinned host batches)."""
+    def train(self, wl, steps, warmup, e2e=True, outputs=False):
+        """value (device-resident inputs), kernel timing, e2e (public KGEModel.train_step on pinned host batches).
+        outputs: also return train_outputs() of the last timed device step (taken before the e2e steps go on)."""
         torch = self.torch
         from knowledgegraphembedding_b200 import KGEModel
         model, nentity, nrel, d, gamma, B, N, lr, de, dr, reg, _ = WORKLOADS[wl]
@@ -399,8 +429,10 @@ class Bench:
                     for p, n, w, md in pool]
         m.train()
 
+        device_out = {}
+
         def step_device(i):
-            m.train_step_async(opt, dev_pool[i % len(dev_pool)], targs)
+            device_out["loss"] = m.train_step_async(opt, dev_pool[i % len(dev_pool)], targs)
 
         m._ws['kernel_events'] = None
         for i in range(warmup):
@@ -413,6 +445,8 @@ class Bench:
                "row_ms": float(np.mean([a.elapsed_time(b) for a, b in events])) if events else None,
                "exchange_ms": float(np.mean([a.elapsed_time(b) for a, b in xevents])) if xevents else None,
                "fused_entity_adam": m.entity_embedding.grad is None, "model": m, "opt": opt, "targs": targs}
+        if outputs:
+            out["outputs"] = train_outputs(m, device_out["loss"])
         px = m._ws.get('peer')
         out["peer"] = px
         out["shard"] = m._ws.get('shard') or None
@@ -496,9 +530,10 @@ class Bench:
         m._ws['eval_events'] = eval_events = []
         self.barrier()
         t0 = time.perf_counter()
+        ranks = {}
         for _ in range(reps):
             for mode in ("head-batch", "tail-batch"):
-                m.filtered_ranks(test, all_true, mode)                 # host triples in, host ranks out
+                ranks[mode] = m.filtered_ranks(test, all_true, mode)   # host triples in, host ranks out
         self.barrier()
         eval_s = (time.perf_counter() - t0) / reps
         m._ws['eval_events'] = None
@@ -509,7 +544,7 @@ class Bench:
                 "cold": {"value": 2 * nq / cold_s, "seconds": cold_s,
                          "what": "first call: python list of all true triples -> int64 array on the host, H2D, filter index built on the device (counting sort)"},
                 "count_kernel_ms": kernel_ms, "count_kernel_queries_per_sec": 2 * nq / (kernel_ms * 1e-3) if kernel_ms else None,
-                "sharding": f"entities/{self.world}", "filter_triples": len(all_true)}, all_true, test
+                "sharding": f"entities/{self.world}", "filter_triples": len(all_true)}, all_true, test, ranks
 
 
 def run_gpu(args):
@@ -520,11 +555,11 @@ def run_gpu(args):
     pk, peak_src = peaks()
     sampler = ClockSampler(b.local)
     sampler.start()
-    tr = b.train(wl, args.steps, args.warmup)
+    tr = b.train(wl, args.steps, args.warmup, outputs=bool(args.dump_outputs) and rank == 0)
     clocks = sampler.stop()
     m = tr["model"]
     De, Dr = m.entity_dim, m.relation_dim
-    ev, all_true, test = b.eval(wl, m, args.eval_queries)
+    ev, all_true, test, eval_ranks = b.eval(wl, m, args.eval_queries)
 
     # ---- the other BASELINE configs (cfg 2, 4, 5), shorter runs ------------------------------------------------------
     extras = {}
@@ -536,11 +571,11 @@ def run_gpu(args):
             if name == wl:
                 continue
             w = WORKLOADS[name]
-            t2 = b.train(name, 10, 3)
+            t2 = b.train(name, args.steps, args.warmup)
             m2 = t2["model"]
             a_tr = train_bytes(w[5], w[6], m2.entity_dim, m2.relation_dim)
             a_ad = adam_bytes(m2.entity_embedding.numel() + m2.relation_embedding.numel())
-            e2, _, _ = b.eval(name, m2, 2048 if name != "rotate_yago310" else 1024, reps=2)
+            e2, _, _, _ = b.eval(name, m2, 2048 if name != "rotate_yago310" else 1024, reps=2)
             entry = {"config": make_config(name, world), "value": t2["value"], "unit": "scores/s",
                      "ms_per_step": t2["ms_per_step"], "e2e": {"value": t2["e2e_value"], "ms_per_step": t2["ms_e2e"]},
                      "fused_entity_adam": t2["fused_entity_adam"],
@@ -680,6 +715,9 @@ def run_gpu(args):
                                                                       + 3 * B * De * 4 / world)) if sh else None)},
         "eval": ev, "workloads": extras,
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {**tr["outputs"], "eval_ranks_head_batch": eval_ranks["head-batch"],
+                                         "eval_ranks_tail_batch": eval_ranks["tail-batch"]})
     emit(line)
     if world > 1:
         b.dist.destroy_process_group()
@@ -710,7 +748,9 @@ def main():
     protect_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed train steps of every GPU workload, at least 1 (the CPU baselines reported beside "
+                         "them keep their own short fixed counts: one reference step takes seconds)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="rotate_fb15k", choices=list(WORKLOADS))
@@ -725,7 +765,15 @@ def main():
     ap.add_argument("--negatives", type=int, default=0, help="experiments: override the workload's negative_sample_size")
     ap.add_argument("--batch", type=int, default=0, help="experiments: override the workload's batch size per GPU")
     ap.add_argument("--entities", type=int, default=0, help="experiments: override the workload's entity count")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="GPU arm, rank 0: after the run, write DIR/<name>.npy (float32/float64, < 64 MB in all) with what "
+                         "the last timed train step returned (train_losses, and the updated tables: entity_embedding is a "
+                         "seeded row sample when it exceeds 28 MB) and the ranks of the last timed evaluation")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU arm computed: it does not apply to --impl reference")
     if args.negatives or args.batch or args.entities:     # (shows up in `config`: not the BASELINE workload any more)
         w = list(WORKLOADS[args.workload])
         w[1], w[5], w[6] = args.entities or w[1], args.batch or w[5], args.negatives or w[6]

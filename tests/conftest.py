@@ -34,6 +34,23 @@ def golden_dir():
     return GOLDEN
 
 
+def load_golden(name):
+    """The arrays of tests/golden/<name>.npz and of its continuation files <name>.2.npz, <name>.3.npz, ...  Golden
+    files are kept under 1 MB each, so a large case is spread over several; an array found in more than one of them
+    is split along its first axis, in file order, and is joined here."""
+    import numpy as np
+    parts, k, path = {}, 1, os.path.join(GOLDEN, name + ".npz")
+    while os.path.exists(path):
+        with np.load(path) as g:
+            for key in g.files:
+                parts.setdefault(key, []).append(g[key])
+        k += 1
+        path = os.path.join(GOLDEN, "%s.%d.npz" % (name, k))
+    if not parts:
+        raise FileNotFoundError(os.path.join(GOLDEN, name + ".npz"))
+    return {key: v[0] if len(v) == 1 else np.concatenate(v) for key, v in parts.items()}
+
+
 def relinf(a, b):
     """max|a-b| / max|b|  (SURVEY section 7 hard part 4: the tolerance is infinity-norm relative)."""
     import numpy as np

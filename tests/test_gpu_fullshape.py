@@ -11,7 +11,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import GOLDEN, outlier_fraction, relinf
+from conftest import GOLDEN, load_golden, outlier_fraction, relinf
 from oracle import c_oracle as C
 from oracle import kge_oracle as O
 from test_gpu_parity import FLAGS, KGE, make_model, ns
@@ -39,7 +39,7 @@ def test_fullwidth_steps_vs_reference_golden(path, monkeypatch):
     if path == "single_read":
         monkeypatch.setenv("KGE_FORCE_SPLIT", "1")
     monkeypatch.setenv("KGE_KEEP_GRADS", "1")
-    g = np.load(os.path.join(GOLDEN, "fullwidth_RotatE_fb15k.npz"))
+    g = load_golden("fullwidth_RotatE_fb15k")
     nentity, nrel, d, gamma = int(g["nentity"]), int(g["nrelation"]), int(g["d"]), float(g["gamma"])
     st = O.init_tables("RotatE", nentity, nrel, d, gamma, True, False, seed=int(g["init_seed"]))
     m = make_model("RotatE", nentity, nrel, d, gamma, st)

@@ -12,7 +12,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import GOLDEN, outlier_fraction, relinf
+from conftest import GOLDEN, load_golden, outlier_fraction, relinf
 from oracle import c_oracle as C
 from oracle import kge_oracle as O
 
@@ -277,7 +277,7 @@ def test_filtered_ranks_vs_reference_golden(model, d):
 
 def test_countries_s1_end_to_end():
     """Real dataset, reference-sampled batches: 4 train steps, AUC-PR (model.py:322-344) and filtered ranks."""
-    g = np.load(os.path.join(GOLDEN, "countries_S1.npz"))
+    g = load_golden("countries_S1")
     d, gamma, nentity, nrel = int(g["d"]), float(g["gamma"]), int(g["nentity"]), int(g["nrelation"])
     from test_oracle_golden import countries_init
     assert (d, g["pos0"].shape[0], g["neg0"].shape[1]) == (500, 512, 64)     # BASELINE configs[0] at its stated shape

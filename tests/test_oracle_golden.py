@@ -5,7 +5,7 @@ import os
 import numpy as np
 import pytest
 
-from conftest import GOLDEN, outlier_fraction, relinf
+from conftest import GOLDEN, load_golden, outlier_fraction, relinf
 from oracle import kge_oracle as O
 
 MODELS = ["TransE", "DistMult", "ComplEx", "RotatE", "pRotatE"]
@@ -157,7 +157,7 @@ def test_fullwidth_reference_golden_pins_both_oracles():
     reference: pins the C oracle -- the full-size checker of the GPU tests and bench.py's CPU port -- at full width,
     and the numpy oracle on the first step."""
     from oracle import c_oracle as C
-    g = np.load(os.path.join(GOLDEN, "fullwidth_RotatE_fb15k.npz"))
+    g = load_golden("fullwidth_RotatE_fb15k")
     nentity, nrel, d, gamma = int(g["nentity"]), int(g["nrelation"]), int(g["d"]), float(g["gamma"])
     st = O.init_tables("RotatE", nentity, nrel, d, gamma, True, False, seed=int(g["init_seed"]))
     assert float(st["entity_embedding"].astype(np.float64).sum()) == float(g["init_checksum"])
@@ -173,7 +173,7 @@ def test_fullwidth_reference_golden_pins_both_oracles():
 
 
 def test_countries_s1_real_dataset():
-    g = np.load(os.path.join(GOLDEN, "countries_S1.npz"))
+    g = load_golden("countries_S1")
     d, gamma = int(g["d"]), float(g["gamma"])
     lr = float(g["lr"])
     ts = O.TrainState("RotatE", countries_init(g), gamma, d)

@@ -1,15 +1,13 @@
 """Negative sampler (SURVEY 8f-1; reference: codes/dataloader.py:13-119,165-186)."""
-import os
-
 import numpy as np
 import pytest
 
-from conftest import GOLDEN
+from conftest import load_golden
 from oracle import kge_oracle as O
 
 
 def countries():
-    g = np.load(os.path.join(GOLDEN, "countries_S1.npz"))
+    g = load_golden("countries_S1")
     tri = [tuple(int(v) for v in r) for r in g["train"]]
     return g, tri, int(g["nentity"]), int(g["nrelation"])
 
