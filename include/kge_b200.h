@@ -269,6 +269,26 @@ int kge_eval_filter_bits_lookup_dense(const int32_t *index_offsets, const int32_
                                       const int64_t *queries, int64_t Q, int mode, int64_t nentity, int64_t nrelation,
                                       uint32_t *filter_bits, void *stream);
 
+/* ---- top-k link prediction: the k most plausible entities of every query (h, r, ?) / (?, r, t) ----
+ * Scores are the canonical exact ones of kge_eval_count_ranks (bit-identical to that kernel and to the C oracle) for
+ * every model; the [Q, nentity] score matrix is never formed.  Order: score descending, then entity id ascending; NaN
+ * after every number; -0.0 == +0.0.  Results travel as uint64 keys (orderable(score) << 32) | (0xFFFFFFFF - id), so a
+ * larger key is a better candidate; key 0 is an empty slot (id -1, score -inf when decoded).
+ * kge_eval_topk: the k best entities in [ent_begin, ent_end) of each query vector (kge_eval_query_vectors; pRotatE also
+ *   needs the phase table) that are not set in exclude_bits ([Q, ceil(nentity/32)] uint32, the filter_bits layout; may
+ *   be NULL).  keys_out [Q, k] sorted best first.  scratch: kge_eval_topk_scratch_bytes() (0 or more; a negative value
+ *   is an error code).  At most 65535*64 queries per call.
+ * kge_eval_topk_merge: the k best of `lists` sorted key lists per query, keys_in [Q, lists, k] (entity shards of several
+ *   devices, say), as keys_out [Q, k] and / or decoded ids_out int64 [Q, k] and scores_out float [Q, k]; each output
+ *   may be NULL.  Keys of one query must be distinct (disjoint entity ranges).                                       */
+#define KGE_TOPK_MAX 256
+int64_t kge_eval_topk_scratch_bytes(const kge_model_t *m, int64_t Q, int64_t ent_begin, int64_t ent_end, int k);
+int kge_eval_topk(const kge_model_t *m, int mode, const float *qvec, int64_t Q, const float *phase_table,
+                  const uint32_t *exclude_bits, int64_t ent_begin, int64_t ent_end, int k, uint64_t *keys_out,
+                  void *scratch, int64_t scratch_bytes, void *stream);
+int kge_eval_topk_merge(const uint64_t *keys_in, int64_t Q, int lists, int k, uint64_t *keys_out, int64_t *ids_out,
+                        float *scores_out, void *stream);
+
 /* ---- negative sampling: TrainDataset.__getitem__ (dataloader.py:28-67) on the device ----
  * For row b (train triple triple_index[b]) draw N entity ids uniformly from the entities that are NOT in the
  * row's sorted true list true_entities[key_start[t] .. +key_len[t])  (the true heads of (r,t) for head-batch, the

@@ -92,7 +92,11 @@ PROTOTYPES = {
                                           c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p,
                                           c_int64, c_void_p, c_void_p, c_void_p]),
     "kge_eval_gemm_band": (c_float, [c_int64]),
-    "kge_sample_negatives": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64, ctypes.c_uint64,
+    "kge_eval_topk_scratch_bytes": (c_int64, [_M, c_int64, c_int64, c_int64, c_int]),
+    "kge_eval_topk": (c_int, [_M, c_int, c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_int64, c_int, c_void_p,
+                              c_void_p, c_int64, c_void_p]),
+    "kge_eval_topk_merge": (c_int, [c_void_p, c_int64, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "kge_sample_negatives":(c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64, ctypes.c_uint64,
                                      ctypes.c_uint64, c_void_p, c_void_p]),
     "kge_eval_filter_bits": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p]),
     "kge_eval_filter_index_scratch_bytes": (c_int64, [c_int64, c_int64]),

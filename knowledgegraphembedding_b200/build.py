@@ -6,9 +6,10 @@ import subprocess
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(CSRC, "libkge_b200.so")
-SOURCES = ["kge_train.cu", "kge_optim.cu", "kge_eval.cu", "kge_eval_gemm.cu", "kge_sampler.cu", "kge_peer.cu",
-           "kge_train_inst.cu"]
-HEADERS = ["kge_common.cuh", "kge_rows.cuh", "kge_adam.cuh", "kge_train_args.cuh", "kge_train_kernels.cuh",
+SOURCES = ["kge_train.cu", "kge_optim.cu", "kge_eval.cu", "kge_eval_gemm.cu", "kge_eval_topk.cu", "kge_sampler.cu",
+           "kge_peer.cu", "kge_train_inst.cu"]
+HEADERS = ["kge_common.cuh", "kge_rows.cuh", "kge_adam.cuh", "kge_eval_tile.cuh", "kge_train_args.cuh",
+           "kge_train_kernels.cuh",
            "kge_train_split.cuh", "kge_train_launch.cuh", "kge_math.h", os.path.join("..", "..", "include", "kge_b200.h")]
 # (source, object suffix, extra flags): the train-path kernels are instantiated once per model (model ids of
 # include/kge_b200.h), one translation unit each, so that the five sets compile in parallel

@@ -1033,6 +1033,97 @@ class KGEModel(nn.Module):
             return ranks, approx
         return (ranks, scores) if return_scores else ranks
 
+    TOPK_MAX = 256          # KGE_TOPK_MAX of include/kge_b200.h
+
+    def predict_topk(self, queries, mode, k=10, exclude_triples=None):
+        """Link prediction: the k most plausible entities for every query, best first.
+
+        queries: (h, r, t) tuples or an int64 array [Q, 3] (the layout of test_triples); mode 'head-batch' predicts h,
+        'tail-batch' predicts t, and the value in the predicted slot is ignored.  exclude_triples: optional list of true
+        triples; every entity that completes a query into one of them is left out (the entity named in the predicted
+        slot included).  Returns (ids int64 [Q, k], scores float32 [Q, k]) on the model's device, ordered by score
+        descending, then entity id ascending; slots beyond the entities left hold id -1 and score -inf.  The scores are
+        the exact ones of the filtered ranking (DESIGN.md section 3.8), for every model.  With an initialised process
+        group every rank selects over its entity slice and the lists are merged (a collective: call it on every rank)."""
+        if mode not in ('head-batch', 'tail-batch'):
+            raise ValueError('negative batch mode %s not supported' % mode)
+        if isinstance(k, bool) or int(k) != k or not 1 <= int(k) <= self.TOPK_MAX:
+            raise ValueError('k must be an integer in [1, %d], got %r' % (self.TOPK_MAX, k))
+        k = int(k)
+        dev = self._device()
+        st = _stream(dev)
+        head = mode == 'head-batch'
+        if isinstance(queries, torch.Tensor):
+            queries_dev = queries.detach().to(device=dev, dtype=torch.int64).reshape(-1, 3).clone()
+            queries_dev[:, 0 if head else 2] = 0
+        else:
+            arr = np.array(queries, dtype=np.int64).reshape(-1, 3)
+            arr[:, 0 if head else 2] = 0         # unused; an out-of-range value would set the bad-index flag
+            queries_dev = torch.from_numpy(arr).to(dev, non_blocking=True)
+        nq = queries_dev.shape[0]
+        ids = torch.empty((nq, k), dtype=torch.int64, device=dev)
+        scores = torch.empty((nq, k), dtype=torch.float32, device=dev)
+        if nq == 0:
+            return ids, scores
+        nentity, nrelation = self.entity_embedding.shape[0], self.relation_embedding.shape[0]
+        ftab = None
+        if exclude_triples is not None:
+            ftab = self._filter_tables(self._filter_index(exclude_triples, nentity, nrelation), mode, dev, st)
+        rank, world = _dist()
+        ent_begin, ent_end = shard_bounds(nentity, rank, world, align=128)
+        desc = self._descriptor()
+        err = self._err_flag()
+        lib = _lib.load()
+        words = (nentity + 31) // 32
+        phase = None
+        if self.model_name == 'pRotatE':
+            phase = self._buffer('phase_table', self.entity_embedding.numel(), torch.float32, dev)
+            _lib.call("kge_eval_phase_table", ctypes.byref(desc), _ptr(phase), st)
+        m = _lib.MODE_IDS[mode]
+        # the keys of this rank's slice, merged over the ranks below (one device: merged and decoded per chunk)
+        local = torch.empty((nq, k), dtype=torch.int64, device=dev) if world > 1 else None
+        chunk = 4096
+        for lo in range(0, nq, chunk):
+            q = queries_dev[lo:lo + chunk]
+            Q = q.shape[0]
+            bits = None
+            if ftab is not None:
+                bits = self._buffer('topk_bits', Q * words, torch.int32, dev)
+                if ftab[0] == 'dense':
+                    _lib.call("kge_eval_filter_bits_lookup_dense", _ptr(ftab[1]), _ptr(ftab[2]), _ptr(q), Q, m, nentity,
+                              nrelation, _ptr(bits), st)
+                else:
+                    _lib.call("kge_eval_filter_bits_lookup", _ptr(ftab[1]), _ptr(ftab[2]), _ptr(ftab[3]), ftab[4],
+                              _ptr(q), Q, m, nentity, nrelation, _ptr(bits), st)
+            qvec = self._buffer('topk_qvec', Q * self.entity_dim, torch.float32, dev)
+            _lib.call("kge_eval_query_vectors", ctypes.byref(desc), m, _ptr(q), Q, _ptr(qvec), _ptr(err), st)
+            sbytes = int(lib.kge_eval_topk_scratch_bytes(ctypes.byref(desc), Q, ent_begin, ent_end, k))
+            _lib.check(min(sbytes, 0))
+            scratch = self._buffer('topk_scratch', sbytes, torch.uint8, dev)
+            keys = local[lo:lo + Q] if local is not None else self._buffer('topk_keys', Q * k, torch.int64, dev)
+            events = self._ws.get('topk_events')             # tools/topk_rate.py: CUDA events around select + merge
+            if events is not None:
+                ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                ev0.record()
+            _lib.call("kge_eval_topk", ctypes.byref(desc), m, _ptr(qvec), Q, _ptr(phase), _ptr(bits), ent_begin,
+                      ent_end, k, _ptr(keys), _ptr(scratch), sbytes, st)
+            if local is None:
+                _lib.call("kge_eval_topk_merge", _ptr(keys), Q, 1, k, None, _ptr(ids[lo:lo + Q]),
+                          _ptr(scores[lo:lo + Q]), st)
+            if events is not None:
+                ev1.record()
+                events.append((ev0, ev1))
+        if local is not None:
+            import torch.distributed as dist
+            gloo = dist.get_backend() == 'gloo'          # gloo gathers host tensors only
+            mine = local.cpu() if gloo else local
+            parts = [torch.empty_like(mine) for _ in range(world)]
+            dist.all_gather(parts, mine)
+            lists = torch.stack(parts, dim=1).to(dev).contiguous()          # [Q, world, k]
+            _lib.call("kge_eval_topk_merge", _ptr(lists), nq, world, k, None, _ptr(ids), _ptr(scores), st)
+        self._raise_if_bad_index()                        # the call's one host sync
+        return ids, scores
+
     @staticmethod
     def test_step(model, test_triples, all_true_triples, args):
         '''
