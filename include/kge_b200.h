@@ -289,6 +289,37 @@ int kge_eval_topk(const kge_model_t *m, int mode, const float *qvec, int64_t Q, 
 int kge_eval_topk_merge(const uint64_t *keys_in, int64_t Q, int lists, int k, uint64_t *keys_out, int64_t *ids_out,
                         float *scores_out, void *stream);
 
+/* ---- relation prediction: which relation links h to t, for every query (h, ?, t) (queries [Q,3] int64, the relation
+ *      slot is the positive for the ranks and is ignored by the top-k) ----
+ * The score of relation r is the 'single'-mode score of (h, r, t) in the canonical order: bit-identical to column t of
+ * the TAIL_BATCH entity scores of (h, r, ?) (kge_eval_count_ranks, kge_eval_topk) and to the C oracle.
+ * kge_eval_relation_table: the relation operand, once per call: rel_table [nrelation, entity_dim] floats = (cos | sin)
+ *   of relation / scale for RotatE, relation / scale for pRotatE; TransE, DistMult and ComplEx use the relation table
+ *   as it is (nothing is written, rel_table may be NULL).  pRotatE also needs kge_eval_phase_table (entity side).
+ * kge_eval_relation_count_ranks: for the relations in [rel_begin, rel_end), counts[q] += #{r != positive, not set in
+ *   filter_bits [Q, ceil(nrelation/32)] : s > s_pos or (s == s_pos and r < positive)} (the tie rule of
+ *   kge_eval_count_ranks).  pos_score from kge_eval_positive_scores in TAIL_BATCH mode on the same queries.
+ *   scores_out [Q, nrelation] (may be NULL) receives the scores of the slice, a filtered column as s_pos - 1.
+ * kge_eval_relation_topk: the k best relations in [rel_begin, rel_end) of each query that are not set in exclude_bits
+ *   (may be NULL), as keys_out [Q, k] in the kge_eval_topk encoding (relation id in the low 32 bits), best first;
+ *   merge the slices of several devices with kge_eval_topk_merge.  scratch: kge_eval_relation_topk_scratch_bytes()
+ *   (0 or more; a negative value is an error code).  An h or t outside the entity table sets *err_flag (may be NULL).
+ * kge_eval_relation_filter_bits: bits [Q, ceil(nrelation/32)] of the relations r with (h, r, t) true, from a sorted-key
+ *   index (keys h*nentity+t int64 [nkeys], run offsets int64 [nkeys+1], relation ids int32).
+ * At most 65535*64 queries per call.                                                                                 */
+int kge_eval_relation_table(const kge_model_t *m, float *rel_table, void *stream);
+int kge_eval_relation_count_ranks(const kge_model_t *m, const int64_t *queries, int64_t Q, const float *rel_table,
+                                  const float *phase_table, const float *pos_score, const uint32_t *filter_bits,
+                                  int64_t rel_begin, int64_t rel_end, int32_t *counts, float *scores_out, void *stream);
+int64_t kge_eval_relation_topk_scratch_bytes(const kge_model_t *m, int64_t Q, int64_t rel_begin, int64_t rel_end, int k);
+int kge_eval_relation_topk(const kge_model_t *m, const int64_t *queries, int64_t Q, const float *rel_table,
+                           const float *phase_table, const uint32_t *exclude_bits, int64_t rel_begin, int64_t rel_end,
+                           int k, uint64_t *keys_out, void *scratch, int64_t scratch_bytes, int32_t *err_flag,
+                           void *stream);
+int kge_eval_relation_filter_bits(const int64_t *index_keys, const int64_t *index_offsets, const int32_t *index_relations,
+                                  int64_t nkeys, const int64_t *queries, int64_t Q, int64_t nentity, int64_t nrelation,
+                                  uint32_t *bits, void *stream);
+
 /* ---- negative sampling: TrainDataset.__getitem__ (dataloader.py:28-67) on the device ----
  * For row b (train triple triple_index[b]) draw N entity ids uniformly from the entities that are NOT in the
  * row's sorted true list true_entities[key_start[t] .. +key_len[t])  (the true heads of (r,t) for head-batch, the

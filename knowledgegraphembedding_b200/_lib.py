@@ -96,6 +96,14 @@ PROTOTYPES = {
     "kge_eval_topk": (c_int, [_M, c_int, c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_int64, c_int, c_void_p,
                               c_void_p, c_int64, c_void_p]),
     "kge_eval_topk_merge": (c_int, [c_void_p, c_int64, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "kge_eval_relation_table": (c_int, [_M, c_void_p, c_void_p]),
+    "kge_eval_relation_count_ranks": (c_int, [_M, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int64,
+                                              c_int64, c_void_p, c_void_p, c_void_p]),
+    "kge_eval_relation_topk_scratch_bytes": (c_int64, [_M, c_int64, c_int64, c_int64, c_int]),
+    "kge_eval_relation_topk": (c_int, [_M, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int,
+                                       c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
+    "kge_eval_relation_filter_bits": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_int64, c_int64,
+                                              c_void_p, c_void_p]),
     "kge_sample_negatives":(c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64, ctypes.c_uint64,
                                      ctypes.c_uint64, c_void_p, c_void_p]),
     "kge_eval_filter_bits": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p]),

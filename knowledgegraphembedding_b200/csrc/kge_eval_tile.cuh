@@ -1,5 +1,6 @@
 // kge_eval_tile.cuh -- the canonical score tile shared by the evaluation kernels (count_ranks_kernel in kge_eval.cu,
-// topk_kernel in kge_eval_topk.cu): element ops, the canonical accumulation order, the cp.async staging of a
+// topk_kernel in kge_eval_topk.cu; relation_tile_kernel in kge_eval_relation.cu reuses the element ops, the constants,
+// the cp.async helpers and the top-k key): element ops, the canonical accumulation order, the cp.async staging of a
 // [64 queries x 64 entities] tile and its k-loop.  Every kernel that runs tile_mainloop<OP, ALIGNED, false> computes the
 // same score bits for a (query, entity) pair, which is what oracle/kge_oracle.c reproduces.
 #pragma once
@@ -232,6 +233,17 @@ __device__ __forceinline__ TileAcc tile_mainloop(const EvalArgs &a, float *smem,
 #pragma unroll
     for (int j = 0; j < 4; ++j) r.v[i][j] = acc[i][j];
   return r;
+}
+
+// Top-k candidate key (kge_eval_topk.cu, kge_eval_relation.cu): (orderable(score) << 32) | (0xFFFFFFFF - id), so that a
+// larger key is a better candidate -- score descending, then id ascending, NaN last, -0.0 == +0.0.  Key 0 is an empty slot.
+__device__ __forceinline__ uint64_t topk_key(float s, int64_t id) {
+  uint32_t ord = 0;                                        // NaN: below every number
+  if (!(s != s)) {
+    const uint32_t u = __float_as_uint(s == 0.f ? 0.f : s);  // -0.0 -> +0.0
+    ord = (u & 0x80000000u) ? ~u : (u | 0x80000000u);     // -inf -> 0x007FFFFF > 0
+  }
+  return ((uint64_t)ord << 32) | (uint64_t)(0xFFFFFFFFu - (uint32_t)id);
 }
 
 static inline int eval_mode(int mode, bool &head) {

@@ -15,15 +15,6 @@
 
 namespace kge {
 
-__device__ __forceinline__ uint64_t topk_key(float s, int64_t id) {
-  uint32_t ord = 0;                                        // NaN: below every number
-  if (!(s != s)) {
-    const uint32_t u = __float_as_uint(s == 0.f ? 0.f : s);  // -0.0 -> +0.0
-    ord = (u & 0x80000000u) ? ~u : (u | 0x80000000u);     // -inf -> 0x007FFFFF > 0
-  }
-  return ((uint64_t)ord << 32) | (uint64_t)(0xFFFFFFFFu - (uint32_t)id);
-}
-
 __device__ __forceinline__ void topk_decode(uint64_t key, int64_t &id, float &score) {
   if (key == 0) {
     id = -1;

@@ -6,6 +6,7 @@ Replaces the per-query python set scan of the reference's TestDataset (codes/dat
     head-batch query (?, r, t)  ->  every h with (h, r, t) true
     tail-batch query (h, r, ?)  ->  every t with (h, r, t) true
 The device turns the lists of one query chunk into the filter bitmap (kge_eval_filter_bits).
+relation_table() is the index of relation prediction, (h, t) -> every r with (h, r, t) true.
 Pure numpy; covered by CPU tests.
 """
 import numpy as np
@@ -66,3 +67,12 @@ class FilterIndex:
         ents = values[idx] if total else np.zeros(0, dtype=np.int32)
         assert run.size == total
         return out_off, np.ascontiguousarray(ents, dtype=np.int32)
+
+
+def relation_table(all_true_triples, nentity):
+    """Relation-prediction index of a list of true triples: (sorted unique keys h*nentity+t int64 [K], run offsets int64
+    [K+1], relation ids int32 [nnz]); run i holds every r with (h, r, t) true for key i.  The key space nentity^2 is too
+    large for a direct-address table, so the keys are sorted and the device looks them up by binary search
+    (kge_eval_relation_filter_bits)."""
+    tri = np.asarray(all_true_triples, dtype=np.int64).reshape(-1, 3)
+    return FilterIndex._group(tri[:, 0] * int(nentity) + tri[:, 2], tri[:, 1])

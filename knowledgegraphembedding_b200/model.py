@@ -17,7 +17,7 @@ import torch
 import torch.nn as nn
 
 from . import _lib
-from .filter_index import FilterIndex
+from .filter_index import FilterIndex, relation_table
 
 _MODELS = ('TransE', 'DistMult', 'ComplEx', 'RotatE', 'pRotatE')
 
@@ -1107,6 +1107,161 @@ class KGEModel(nn.Module):
                 ev0.record()
             _lib.call("kge_eval_topk", ctypes.byref(desc), m, _ptr(qvec), Q, _ptr(phase), _ptr(bits), ent_begin,
                       ent_end, k, _ptr(keys), _ptr(scratch), sbytes, st)
+            if local is None:
+                _lib.call("kge_eval_topk_merge", _ptr(keys), Q, 1, k, None, _ptr(ids[lo:lo + Q]),
+                          _ptr(scores[lo:lo + Q]), st)
+            if events is not None:
+                ev1.record()
+                events.append((ev0, ev1))
+        if local is not None:
+            import torch.distributed as dist
+            gloo = dist.get_backend() == 'gloo'          # gloo gathers host tensors only
+            mine = local.cpu() if gloo else local
+            parts = [torch.empty_like(mine) for _ in range(world)]
+            dist.all_gather(parts, mine)
+            lists = torch.stack(parts, dim=1).to(dev).contiguous()          # [Q, world, k]
+            _lib.call("kge_eval_topk_merge", _ptr(lists), nq, world, k, None, _ptr(ids), _ptr(scores), st)
+        self._raise_if_bad_index()                        # the call's one host sync
+        return ids, scores
+
+    # ------------------------------------------------------------------------------------------ relation prediction
+    def _relation_filter_table(self, held, dev):
+        """The relation index h*nentity+t -> relations of one true-triple list (filter_index.relation_table), resident on
+        the device: built on the first relation request and kept in the list's _filter_cache entry next to the entity
+        tables, which never pay for it."""
+        tab = held['tables'].get(('relation', dev))
+        if tab is None:
+            keys, offsets, values = relation_table(held['list'], held['key'][1])
+            tab = (torch.from_numpy(keys).to(dev), torch.from_numpy(offsets).to(dev),
+                   torch.from_numpy(values).to(dev) if values.size else torch.zeros(1, dtype=torch.int32, device=dev),
+                   int(keys.size))
+            held['tables'][('relation', dev)] = tab
+        return tab
+
+    def _relation_operands(self, desc, dev, st):
+        """(relation operand table, phase table) of kge_eval_relation_*: the table for RotatE / pRotatE, the phase table
+        for pRotatE, None otherwise.  (The phase table is the buffer of filtered_ranks / predict_topk: same size, same
+        values.)"""
+        rel_table = phase = None
+        if self.model_name in ('RotatE', 'pRotatE'):
+            rel_table = self._buffer('rel_operand', self.relation_embedding.shape[0] * self.entity_dim, torch.float32, dev)
+            _lib.call("kge_eval_relation_table", ctypes.byref(desc), _ptr(rel_table), st)
+        if self.model_name == 'pRotatE':
+            phase = self._buffer('phase_table', self.entity_embedding.numel(), torch.float32, dev)
+            _lib.call("kge_eval_phase_table", ctypes.byref(desc), _ptr(phase), st)
+        return rel_table, phase
+
+    def filtered_relation_ranks(self, test_triples, all_true_triples, query_chunk=4096, return_scores=False):
+        """Filtered relation rank of every test triple (h, r, t) among all relations for the query (h, ?, t): int64 [len],
+        1 + #{r' != r unfiltered: s(h,r',t) > s(h,r,t)} + #{r' < r unfiltered: equal score}, where r' is filtered when
+        (h, r', t) is in all_true_triples.  s is the exact 'single'-mode score (DESIGN.md section 3.9); metrics_from_ranks
+        turns the ranks into MRR / Hits@k.  return_scores: also the [len, nrelation] scores (a filtered column holds
+        s(h,r,t) - 1).  With an initialised process group every rank counts over its relation slice and the counts are
+        all-reduced (a collective: call it on every rank)."""
+        dev = self._device()
+        st = _stream(dev)
+        nentity, nrelation = self.entity_embedding.shape[0], self.relation_embedding.shape[0]
+        queries_all = np.asarray(test_triples, dtype=np.int64).reshape(-1, 3)
+        nq = queries_all.shape[0]
+        queries_dev = torch.from_numpy(queries_all).to(dev, non_blocking=True)
+        ftab = self._relation_filter_table(self._filter_index(all_true_triples, nentity, nrelation), dev)
+        rank, world = _dist()
+        rel_begin, rel_end = shard_bounds(nrelation, rank, world, align=64)
+        desc = self._descriptor()
+        err = self._err_flag()
+        rel_table, phase = self._relation_operands(desc, dev, st)
+        words = (nrelation + 31) // 32
+        counts_all = torch.zeros(max(nq, 1), dtype=torch.int32, device=dev)
+        scores = torch.empty((nq, nrelation), dtype=torch.float32, device=dev) if return_scores else None
+        tail = _lib.MODE_IDS['tail-batch']
+        for lo in range(0, nq, query_chunk):
+            queries = queries_dev[lo:lo + query_chunk]
+            Q = queries.shape[0]
+            bits = self._buffer('rel_filter_bits', Q * words, torch.int32, dev)
+            qvec = self._buffer('rel_qvec', Q * self.entity_dim, torch.float32, dev)
+            pos = self._buffer('rel_pos_score', Q, torch.float32, dev)
+            _lib.call("kge_eval_relation_filter_bits", _ptr(ftab[0]), _ptr(ftab[1]), _ptr(ftab[2]), ftab[3],
+                      _ptr(queries), Q, nentity, nrelation, _ptr(bits), st)
+            # s(h, r, t) of the positive: the tail-batch query vector and positive score, the same fold, op and order
+            _lib.call("kge_eval_query_vectors", ctypes.byref(desc), tail, _ptr(queries), Q, _ptr(qvec), _ptr(err), st)
+            _lib.call("kge_eval_positive_scores", ctypes.byref(desc), tail, _ptr(qvec), _ptr(queries), Q, _ptr(phase),
+                      _ptr(pos), st)
+            events = self._ws.get('relation_events')         # tools/relation_rate.py: CUDA events around the kernel
+            if events is not None:
+                ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                ev0.record()
+            _lib.call("kge_eval_relation_count_ranks", ctypes.byref(desc), _ptr(queries), Q, _ptr(rel_table), _ptr(phase),
+                      _ptr(pos), _ptr(bits), rel_begin, rel_end, _ptr(counts_all[lo:lo + Q]),
+                      _ptr(scores[lo:lo + Q]) if scores is not None else None, st)
+            if events is not None:
+                ev1.record()
+                events.append((ev0, ev1))
+        if world > 1:
+            import torch.distributed as dist
+            if dist.get_backend() == 'gloo':
+                counts_all = counts_all.cpu()
+            dist.all_reduce(counts_all)                      # integer sums over the relation slices: bit-exact
+        ranks = counts_all.cpu().numpy()[:nq].astype(np.int64) + 1      # the call's one host sync
+        self._raise_if_bad_index()
+        return (ranks, scores) if return_scores else ranks
+
+    def predict_relations(self, queries, k=10, exclude_triples=None):
+        """Relation prediction: the k most plausible relations r for every query (h, ?, t), best first.
+
+        queries: (h, r, t) tuples or an int64 array [Q, 3] (the layout of test_triples); the relation slot is ignored.
+        exclude_triples: optional list of true triples; every r with (h, r, t) in it is left out.  Returns (ids int64
+        [Q, k], scores float32 [Q, k]) on the model's device, ordered as predict_topk's: score descending, then relation
+        id ascending, NaN last; slots beyond the relations left hold id -1 and score -inf (k may exceed nrelation).  The
+        scores are the exact ones of filtered_relation_ranks.  With an initialised process group every rank selects over
+        its relation slice and the lists are merged (a collective: call it on every rank)."""
+        if isinstance(k, bool) or int(k) != k or not 1 <= int(k) <= self.TOPK_MAX:
+            raise ValueError('k must be an integer in [1, %d], got %r' % (self.TOPK_MAX, k))
+        k = int(k)
+        dev = self._device()
+        st = _stream(dev)
+        if isinstance(queries, torch.Tensor):
+            queries_dev = queries.detach().to(device=dev, dtype=torch.int64).reshape(-1, 3).clone()
+            queries_dev[:, 1] = 0
+        else:
+            arr = np.array(queries, dtype=np.int64).reshape(-1, 3)
+            arr[:, 1] = 0
+            queries_dev = torch.from_numpy(arr).to(dev, non_blocking=True)
+        nq = queries_dev.shape[0]
+        ids = torch.empty((nq, k), dtype=torch.int64, device=dev)
+        scores = torch.empty((nq, k), dtype=torch.float32, device=dev)
+        if nq == 0:
+            return ids, scores
+        nentity, nrelation = self.entity_embedding.shape[0], self.relation_embedding.shape[0]
+        ftab = None
+        if exclude_triples is not None:
+            ftab = self._relation_filter_table(self._filter_index(exclude_triples, nentity, nrelation), dev)
+        rank, world = _dist()
+        rel_begin, rel_end = shard_bounds(nrelation, rank, world, align=64)
+        desc = self._descriptor()
+        err = self._err_flag()
+        lib = _lib.load()
+        rel_table, phase = self._relation_operands(desc, dev, st)
+        words = (nrelation + 31) // 32
+        local = torch.empty((nq, k), dtype=torch.int64, device=dev) if world > 1 else None
+        chunk = 4096
+        for lo in range(0, nq, chunk):
+            q = queries_dev[lo:lo + chunk]
+            Q = q.shape[0]
+            bits = None
+            if ftab is not None:
+                bits = self._buffer('rel_topk_bits', Q * words, torch.int32, dev)
+                _lib.call("kge_eval_relation_filter_bits", _ptr(ftab[0]), _ptr(ftab[1]), _ptr(ftab[2]), ftab[3], _ptr(q),
+                          Q, nentity, nrelation, _ptr(bits), st)
+            sbytes = int(lib.kge_eval_relation_topk_scratch_bytes(ctypes.byref(desc), Q, rel_begin, rel_end, k))
+            _lib.check(min(sbytes, 0))
+            scratch = self._buffer('rel_topk_scratch', sbytes, torch.uint8, dev)
+            keys = local[lo:lo + Q] if local is not None else self._buffer('rel_topk_keys', Q * k, torch.int64, dev)
+            events = self._ws.get('relation_topk_events')    # tools/relation_rate.py: CUDA events around select + merge
+            if events is not None:
+                ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                ev0.record()
+            _lib.call("kge_eval_relation_topk", ctypes.byref(desc), _ptr(q), Q, _ptr(rel_table), _ptr(phase), _ptr(bits),
+                      rel_begin, rel_end, k, _ptr(keys), _ptr(scratch), sbytes, _ptr(err), st)
             if local is None:
                 _lib.call("kge_eval_topk_merge", _ptr(keys), Q, 1, k, None, _ptr(ids[lo:lo + Q]),
                           _ptr(scores[lo:lo + Q]), st)
