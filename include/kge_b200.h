@@ -220,6 +220,19 @@ int kge_eval_count_ranks_two_stage(const kge_model_t *m, int mode, const float *
                                    const uint32_t *filter_bits, int64_t ent_begin, int64_t ent_end,
                                    int32_t *counts, void *amb_pairs, int64_t amb_capacity, int32_t *amb_count,
                                    void *stream);
+/* The same, and approx_scores_out (tests, may be NULL): [Q, nentity] dump, for the entities in [ent_begin, ent_end), of the
+ * score each pair was decided on -- the fast pass's approximation (a filtered column as s_pos - 1; NaN where the pRotatE
+ * pass gives up), or the exact score where the exact kernel runs instead (no fast variant, d > 2048, unaligned rows).
+ * A fast pass zeroes amb_count; the exact kernel leaves it untouched.                                              */
+int kge_eval_count_ranks_two_stage_approx(const kge_model_t *m, int mode, const float *qvec, const int64_t *queries,
+                                          int64_t Q, const float *phase_table, const float *pos_score,
+                                          const uint32_t *filter_bits, int64_t ent_begin, int64_t ent_end,
+                                          int32_t *counts, void *amb_pairs, int64_t amb_capacity, int32_t *amb_count,
+                                          float *approx_scores_out, void *stream);
+/* The band of the fast pass (what the band test in tests/ pins): |approx - canonical| <= eps(approx) =
+ * host_band[0] + host_band[1] * |gamma - approx| + host_band[2] * |approx| for `model` (KGE_ROTATE / KGE_PROTATE), its
+ * entity_dim and (pRotatE) modulus.  KGE_ERR_INVALID for a model or entity_dim without a fast pass.               */
+int kge_eval_two_stage_band(int model, int64_t entity_dim, float modulus, float *host_band);
 
 /* ---- tcgen05 path for the dot-product models (DistMult model.py:175-182, ComplEx :184-199) in test_step ----
  * The all-entity scores are one [Q, D_e] x [D_e, nentity] contraction.  Operands are split into two TF32-exact

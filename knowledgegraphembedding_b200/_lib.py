@@ -86,6 +86,10 @@ PROTOTYPES = {
                                      c_int64, c_void_p, c_void_p, c_void_p]),
     "kge_eval_count_ranks_two_stage": (c_int, [_M, c_int, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p,
                                                c_int64, c_int64, c_void_p, c_void_p, c_int64, c_void_p, c_void_p]),
+    "kge_eval_count_ranks_two_stage_approx": (c_int, [_M, c_int, c_void_p, c_void_p, c_int64, c_void_p, c_void_p,
+                                                      c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_int64, c_void_p,
+                                                      c_void_p, c_void_p]),
+    "kge_eval_two_stage_band": (c_int, [c_int, c_int64, c_float, POINTER(c_float)]),
     "kge_eval_gemm_supported": (c_int, [_M]),
     "kge_eval_gemm_split": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_void_p]),
     "kge_eval_gemm_count_ranks": (c_int, [_M, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p,

@@ -109,6 +109,7 @@ __global__ void __launch_bounds__(EVAL_THREADS, 2) count_ranks_kernel(const Eval
 
   // ---- epilogue: compare with the positive, apply the filter, count -------------------------------------------
   const float modulus = a.modulus ? a.modulus[0] : 1.f;
+  [[maybe_unused]] const FastBand band = fast_band(OP != OP_CDIST, a.d, modulus);
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
     const int64_t qi = q0 + tq + 16 * i;
@@ -125,9 +126,7 @@ __global__ void __launch_bounds__(EVAL_THREADS, 2) count_ranks_kernel(const Eval
       if (filtered) s = fadd(sp, -1.0f);                   // candidate replaced by the positive, bias -1
       else if (ej != pid) {
         if constexpr (FAST) {                              // s is only within eps of the canonical score
-          float eps;
-          if constexpr (OP == OP_CDIST) eps = kFastBand * (a.gamma - s) + 1e-12f;
-          else eps = fabsf(modulus) * (float)a.d * kFastSinTerm + kFastSinSum * fabsf(a.gamma - s) + 1e-12f;
+          const float eps = fast_eps(band, a.gamma, s);
           if (s - eps > sp) ++c;
           else if (!(s + eps < sp)) {                      // undecidable here (or NaN): exact re-score later
             const int slot = atomicAdd(a.amb_count, 1);
@@ -270,7 +269,7 @@ static int launch_count(const EvalArgs &a, bool aligned, cudaStream_t st) {
   const size_t smem = sizeof(float) * 2 * (TQ + TJ) * H * ST;
   dim3 grid((unsigned)((a.ent_end - a.ent_begin + TJ - 1) / TJ), (unsigned)((a.Q + TQ - 1) / TQ));
   if constexpr (OP == OP_CDIST || OP == OP_SUBSIN || OP == OP_ADDSIN) {
-    if (a.amb && aligned && !a.scores_out && a.d <= 2048) {          // two-stage: fast tile pass + exact re-score
+    if (a.amb && aligned && a.d <= kFastMaxD) {                      // two-stage: fast tile pass + exact re-score
       KGE_CUDA_OK(cudaMemsetAsync(a.amb_count, 0, 2 * sizeof(int), st));
       auto k = count_ranks_kernel<OP, true, true>;
       KGE_CUDA_OK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -395,9 +394,33 @@ extern "C" int kge_eval_count_ranks_two_stage(const kge_model_t *m, int mode, co
                                               const uint32_t *filter_bits, int64_t ent_begin, int64_t ent_end,
                                               int32_t *counts, void *amb_pairs, int64_t amb_capacity,
                                               int32_t *amb_count, void *stream) {
+  return kge_eval_count_ranks_two_stage_approx(m, mode, qvec, queries, Q, phase_table, pos_score, filter_bits, ent_begin,
+                                               ent_end, counts, amb_pairs, amb_capacity, amb_count, nullptr, stream);
+}
+
+extern "C" int kge_eval_count_ranks_two_stage_approx(const kge_model_t *m, int mode, const float *qvec,
+                                                     const int64_t *queries, int64_t Q, const float *phase_table,
+                                                     const float *pos_score, const uint32_t *filter_bits,
+                                                     int64_t ent_begin, int64_t ent_end, int32_t *counts,
+                                                     void *amb_pairs, int64_t amb_capacity, int32_t *amb_count,
+                                                     float *approx_scores_out, void *stream) {
   KGE_REQUIRE(amb_pairs && amb_count && amb_capacity > 0, "two-stage ranking needs the ambiguous-pair buffers");
+  // the fast pass writes its own scores through scores_out (only this entry sets both scores_out and the pair list)
   return count_ranks_impl(m, mode, qvec, queries, Q, phase_table, pos_score, filter_bits, ent_begin, ent_end, counts,
-                          nullptr, amb_pairs, amb_capacity, amb_count, stream);
+                          approx_scores_out, amb_pairs, amb_capacity, amb_count, stream);
+}
+
+extern "C" int kge_eval_two_stage_band(int model, int64_t entity_dim, float modulus, float *host_band) {
+  KGE_REQUIRE(host_band, "null pointer");
+  KGE_REQUIRE(model == KGE_ROTATE || model == KGE_PROTATE, "model %d has no two-stage pass", model);
+  const int64_t d = model == KGE_ROTATE ? entity_dim / 2 : entity_dim;
+  KGE_REQUIRE(entity_dim > 0 && (model != KGE_ROTATE || entity_dim % 2 == 0) && d <= kFastMaxD,
+              "entity_dim %lld has no two-stage pass (d at most %d)", (long long)entity_dim, kFastMaxD);
+  const FastBand b = fast_band(model == KGE_PROTATE, (int)d, modulus);
+  host_band[0] = b.c_abs;
+  host_band[1] = b.c_rel;
+  host_band[2] = b.c_ulp;
+  return KGE_OK;
 }
 
 static int count_ranks_impl(const kge_model_t *m, int mode, const float *qvec, const int64_t *queries, int64_t Q,

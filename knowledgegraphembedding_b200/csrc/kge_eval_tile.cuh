@@ -48,11 +48,33 @@ __device__ __forceinline__ float op_fast(float q0, float q1, float x0, float x1)
   } else if constexpr (OP == OP_SUBSIN) return abs_sin_fast(q0 - x0);
   else return abs_sin_fast(x0 + q0);
 }
-// |s_fast - s_canonical| <= kFastBand * (gamma - s_fast): 2^-20 per term + two blocked fp32 sums of the same
-// blocks (each within (32 + d/32) * 2^-24 <= 6e-6 of the exact sum for d <= 2048), rounded up.
+// Band of the two-stage pass: |s_fast - s_canonical| <= eps(s_fast) = c_abs + c_rel * |gamma - s_fast| + c_ulp * |s_fast|
+// (fast_band / fast_eps below; kge_eval_two_stage_band exports the coefficients).  Both scores are
+// s = fl(gamma - p), p = acc (RotatE) or fl(acc * modulus) (pRotatE), of two different sums acc_f and acc_c.
+//  * c_rel, the sums.  RotatE: 2^-20 per term + two blocked fp32 sums of the same blocks (each within (32 + d/32) * 2^-24
+//    <= 6e-6 of the exact sum for d <= 2048), rounded up: kFastBand.  pRotatE: the same two sums (1.15e-5) and the two
+//    roundings of acc * modulus (1.2e-7) fit in kFastSinSum; its per-term error is absolute, c_abs = |modulus| d kFastSinTerm.
+//  * c_ulp, the final subtraction.  fl(x) = x (1 + e) with |e| <= 2^-24 gives |s - (gamma - p)| <= 2^-24 |s| for s_f and
+//    for s_c, and |s_c| <= |s_f| + eps, so the two roundings add 2^-23 |s_f| (+ 2^-24 eps, second order).  This term does
+//    not shrink with |p_f - p_c|: sums that straddle a rounding boundary of gamma - p give scores one ulp of s apart however
+//    close they are, while c_rel * |gamma - s| falls below that ulp once acc < ulp(gamma) / c_rel (0.12 at gamma = 24).
+//    kFastUlp = 2^-22 takes it twice: the margin covers |gamma - s_f| underestimating |p_f| by up to 2^-24 |s_f| (times
+//    c_rel) and the fp32 evaluation of eps (a few ulps of eps).
 constexpr float kFastBand = 1.6e-5f;
 // pRotatE: per term |fast - canonical| <= 5.1e-7 + 1.04e-6 (above) + 1.8e-7 (sin_rep's own 1.5 ulp) < kFastSinTerm; sums as above
 constexpr float kFastSinTerm = 2.0e-6f, kFastSinSum = 1.2e-5f;
+constexpr float kFastUlp = 0x1p-22f;
+constexpr int kFastMaxD = 2048;                            // the sum bounds above hold up to this d
+struct FastBand {
+  float c_abs, c_rel, c_ulp;
+};
+KGE_HD FastBand fast_band(bool protate, int d, float modulus) {
+  if (protate) return FastBand{fabsf(modulus) * (float)d * kFastSinTerm + 1e-12f, kFastSinSum, kFastUlp};
+  return FastBand{1e-12f, kFastBand, kFastUlp};
+}
+KGE_HD float fast_eps(const FastBand &b, float gamma, float s) {
+  return b.c_abs + b.c_rel * fabsf(gamma - s) + b.c_ulp * fabsf(s);
+}
 
 template <int OP>
 __device__ __forceinline__ float finish_exact(float acc, float gamma, float modulus) {
@@ -83,7 +105,7 @@ struct EvalArgs {
   const float *pos_score;       // [Q]
   const uint32_t *filter_bits;  // [Q, words]
   int32_t *counts;              // [Q]
-  float *scores_out;            // [Q, nentity] or null
+  float *scores_out;            // [Q, nentity] or null: the score each pair was decided on (the fast one in a FAST pass)
   const float *modulus;
   int64_t Q, nentity, ent_begin, ent_end;
   int d, De, pos_col, words;

@@ -968,8 +968,10 @@ class KGEModel(nn.Module):
                       _ptr(enorm), st)
         counts_all = tally[:nq_all]
         scores = torch.empty((queries_all.shape[0], nentity), dtype=torch.float32, device=dev) if return_scores else None
-        # tests: the tensor-core approximations of the tcgen05 path (to pin its error band against exact scores)
-        approx = torch.zeros((queries_all.shape[0], nentity), dtype=torch.float32, device=dev) if (return_approx and gemm) else None
+        # tests: the approximations of the tcgen05 path or of the two-stage fast pass (to pin their error bands against
+        # exact scores)
+        approx = torch.zeros((queries_all.shape[0], nentity), dtype=torch.float32, device=dev) \
+            if (return_approx and (gemm or two_stage)) else None
         m = _lib.MODE_IDS[mode]
         for ci, lo in enumerate(range(0, queries_all.shape[0], query_chunk)):
             queries = queries_dev[lo:lo + query_chunk]
@@ -1006,9 +1008,9 @@ class KGEModel(nn.Module):
             elif two_stage:
                 cap = int(os.environ.get('KGE_EVAL_AMB_CAP', Q * 256))
                 amb = self._buffer('gemm_amb', cap * 2, torch.int32, dev)
-                _lib.call("kge_eval_count_ranks_two_stage", ctypes.byref(desc), m, _ptr(qvec), _ptr(queries), Q,
+                _lib.call("kge_eval_count_ranks_two_stage_approx", ctypes.byref(desc), m, _ptr(qvec), _ptr(queries), Q,
                           _ptr(phase), _ptr(pos), _ptr(bits), ent_begin, ent_end, _ptr(counts), _ptr(amb), cap,
-                          _ptr(amb_counts[ci]), st)
+                          _ptr(amb_counts[ci]), _ptr(approx[lo:lo + Q]) if approx is not None else None, st)
             else:
                 _lib.call("kge_eval_count_ranks", ctypes.byref(desc), m, _ptr(qvec), _ptr(queries), Q, _ptr(phase),
                           _ptr(pos), _ptr(bits), ent_begin, ent_end, _ptr(counts),
