@@ -254,6 +254,33 @@ int kge_eval_gemm_count_ranks(const kge_model_t *m, int mode, const float *qvec,
  * of the tensor-core approximations for the entities in [ent_begin, ent_end).                                    */
 float kge_eval_gemm_band(int64_t entity_dim);
 
+/* ---- rank statistics: raw and tie-aware ranks from the same passes ----
+ * The three step-3 entries above, counting KGE_RANK_STATS int32 counters per query instead of one:
+ * stats [Q, KGE_RANK_STATS], zeroed by the caller; for the entities j != pos(q) in [ent_begin, ent_end), with s the
+ * canonical score of kge_eval_count_ranks (a filtered column keeps its own score here) and "filtered" read from
+ * filter_bits:
+ *   [0] !filtered && s > s_pos            [3] s > s_pos
+ *   [1] !filtered && s == s_pos && j < pos  [4] s == s_pos && j < pos
+ *   [2] !filtered && s == s_pos && j > pos  [5] s == s_pos && j > pos
+ * NaN is never greater or equal, -0.0 == +0.0, and the counters add up over entity slices.  1 + [0] + [1] is the rank of
+ * kge_eval_count_ranks whenever fl(s_pos - 1) < s_pos (the filter bias of that rank); 1 + [3] + [4] is the raw rank.
+ * The two-stage and tcgen05 variants take the argument rules of their count entries (amb_count[1] = 1: overflow, the
+ * caller re-runs kge_eval_count_rank_stats for that chunk; ent_begin a multiple of 32 on tcgen05).              */
+#define KGE_RANK_STATS 6
+int kge_eval_count_rank_stats(const kge_model_t *m, int mode, const float *qvec, const int64_t *queries, int64_t Q,
+                              const float *phase_table, const float *pos_score, const uint32_t *filter_bits,
+                              int64_t ent_begin, int64_t ent_end, int32_t *stats, void *stream);
+int kge_eval_count_rank_stats_two_stage(const kge_model_t *m, int mode, const float *qvec, const int64_t *queries,
+                                        int64_t Q, const float *phase_table, const float *pos_score,
+                                        const uint32_t *filter_bits, int64_t ent_begin, int64_t ent_end, int32_t *stats,
+                                        void *amb_pairs, int64_t amb_capacity, int32_t *amb_count, void *stream);
+int kge_eval_gemm_count_rank_stats(const kge_model_t *m, int mode, const float *qvec, const float *qhi,
+                                   const float *qlo, const float *qnorm, const int64_t *queries, int64_t Q,
+                                   const float *pos_score, const uint32_t *filter_bits, const float *ehi,
+                                   const float *elo, const float *enorm, int64_t ent_begin, int64_t ent_end,
+                                   int32_t *stats, void *amb_pairs, int64_t amb_capacity, int32_t *amb_count,
+                                   void *stream);
+
 /* filter bitmap from a CSR of true entities per query (dataloader.py:138-144)                     */
 int kge_eval_filter_bits(const int64_t *csr_offsets, const int32_t *csr_entities, int64_t Q,
                          int64_t nentity, uint32_t *filter_bits, void *stream);

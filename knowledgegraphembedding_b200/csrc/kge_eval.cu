@@ -93,56 +93,105 @@ __global__ void positive_scores_kernel(const float *__restrict__ qvec, const flo
 }
 
 // ---- tiled score + count ---------------------------------------------------------------------------------------
-template <int OP, bool ALIGNED, bool FAST = false>
+// STATS: a.counts is the [Q, KGE_RANK_STATS] table of kge_eval_count_rank_stats instead of [Q] counts.
+template <int OP, bool ALIGNED, bool FAST = false, bool STATS = false>
 __global__ void __launch_bounds__(EVAL_THREADS, 2) count_ranks_kernel(const EvalArgs a) {
   extern __shared__ __align__(16) float smem[];
-  __shared__ int cnt_sh[TQ];
+  __shared__ int cnt_sh[STATS ? KGE_RANK_STATS * TQ : TQ];
 
   const int tid = threadIdx.x;
   const int tq = tid % 16, tj = tid / 16;
   const int64_t j0 = a.ent_begin + (int64_t)blockIdx.x * TJ;
   const int64_t q0 = (int64_t)blockIdx.y * TQ;
-  if (tid < TQ) cnt_sh[tid] = 0;
+  if constexpr (STATS) {
+    for (int i = tid; i < KGE_RANK_STATS * TQ; i += EVAL_THREADS) cnt_sh[i] = 0;
+  } else {
+    if (tid < TQ) cnt_sh[tid] = 0;
+  }
 
   const TileAcc t = tile_mainloop<OP, ALIGNED, FAST>(a, smem, q0, j0, tq, tj);
   const auto &acc = t.v;
 
-  // ---- epilogue: compare with the positive, apply the filter, count -------------------------------------------
   const float modulus = a.modulus ? a.modulus[0] : 1.f;
   [[maybe_unused]] const FastBand band = fast_band(OP != OP_CDIST, a.d, modulus);
+  if constexpr (STATS) {
+    // ---- epilogue: the six counters of every column but the positive's; a filtered column keeps its own score ----
 #pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int64_t qi = q0 + tq + 16 * i;
-    if (qi >= a.Q) continue;
-    const float sp = a.pos_score[qi];
-    int64_t pid = a.queries[qi * 3 + a.pos_col];
-    int c = 0;
+    for (int i = 0; i < 4; ++i) {
+      const int64_t qi = q0 + tq + 16 * i;
+      if (qi >= a.Q) continue;
+      const float sp = a.pos_score[qi];
+      const int64_t pid = a.queries[qi * 3 + a.pos_col];
+      int c[KGE_RANK_STATS] = {0, 0, 0, 0, 0, 0};
 #pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const int64_t ej = j0 + tj + 16 * j;
-      if (ej >= a.ent_end) continue;
-      float s = finish_exact<OP>(acc[i][j], a.gamma, modulus);
-      const bool filtered = ej != pid && ((a.filter_bits[qi * a.words + (ej >> 5)] >> (ej & 31)) & 1u);
-      if (filtered) s = fadd(sp, -1.0f);                   // candidate replaced by the positive, bias -1
-      else if (ej != pid) {
-        if constexpr (FAST) {                              // s is only within eps of the canonical score
+      for (int j = 0; j < 4; ++j) {
+        const int64_t ej = j0 + tj + 16 * j;
+        if (ej >= a.ent_end || ej == pid) continue;
+        const float s = finish_exact<OP>(acc[i][j], a.gamma, modulus);
+        const bool kept = !((a.filter_bits[qi * a.words + (ej >> 5)] >> (ej & 31)) & 1u);
+        if constexpr (FAST) {                            // s is only within eps of the canonical score
           const float eps = fast_eps(band, a.gamma, s);
-          if (s - eps > sp) ++c;
-          else if (!(s + eps < sp)) {                      // undecidable here (or NaN): exact re-score later
+          if (s - eps > sp) {
+            c[0] += kept;
+            ++c[3];
+          } else if (!(s + eps < sp)) {                  // equal, undecidable here, or NaN: exact re-score later
             const int slot = atomicAdd(a.amb_count, 1);
             if (slot < a.amb_capacity) a.amb[slot] = make_int2((int)qi, (int)ej);
             else a.amb_count[1] = 1;
           }
         } else {
-          c += (s > sp) || (s == sp && ej < pid);
+          const bool gt = s > sp, eb = s == sp && ej < pid, ea = s == sp && ej > pid;
+          c[0] += kept && gt;
+          c[1] += kept && eb;
+          c[2] += kept && ea;
+          c[3] += gt;
+          c[4] += eb;
+          c[5] += ea;
         }
       }
-      if (a.scores_out) a.scores_out[qi * a.nentity + ej] = s;
+#pragma unroll
+      for (int k = 0; k < KGE_RANK_STATS; ++k)
+        if (c[k]) atomicAdd(&cnt_sh[(tq + 16 * i) * KGE_RANK_STATS + k], c[k]);
     }
-    if (c) atomicAdd(&cnt_sh[tq + 16 * i], c);
+    __syncthreads();
+    for (int i = tid; i < KGE_RANK_STATS * TQ; i += EVAL_THREADS)
+      if (cnt_sh[i] && q0 + i / KGE_RANK_STATS < a.Q) atomicAdd(&a.counts[q0 * KGE_RANK_STATS + i], cnt_sh[i]);
+  } else {
+    // ---- epilogue: compare with the positive, apply the filter, count -------------------------------------------
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      const int64_t qi = q0 + tq + 16 * i;
+      if (qi >= a.Q) continue;
+      const float sp = a.pos_score[qi];
+      int64_t pid = a.queries[qi * 3 + a.pos_col];
+      int c = 0;
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const int64_t ej = j0 + tj + 16 * j;
+        if (ej >= a.ent_end) continue;
+        float s = finish_exact<OP>(acc[i][j], a.gamma, modulus);
+        const bool filtered = ej != pid && ((a.filter_bits[qi * a.words + (ej >> 5)] >> (ej & 31)) & 1u);
+        if (filtered) s = fadd(sp, -1.0f);                   // candidate replaced by the positive, bias -1
+        else if (ej != pid) {
+          if constexpr (FAST) {                              // s is only within eps of the canonical score
+            const float eps = fast_eps(band, a.gamma, s);
+            if (s - eps > sp) ++c;
+            else if (!(s + eps < sp)) {                      // undecidable here (or NaN): exact re-score later
+              const int slot = atomicAdd(a.amb_count, 1);
+              if (slot < a.amb_capacity) a.amb[slot] = make_int2((int)qi, (int)ej);
+              else a.amb_count[1] = 1;
+            }
+          } else {
+            c += (s > sp) || (s == sp && ej < pid);
+          }
+        }
+        if (a.scores_out) a.scores_out[qi * a.nentity + ej] = s;
+      }
+      if (c) atomicAdd(&cnt_sh[tq + 16 * i], c);
+    }
+    __syncthreads();
+    if (tid < TQ && cnt_sh[tid] && q0 + tid < a.Q) atomicAdd(&a.counts[q0 + tid], cnt_sh[tid]);
   }
-  __syncthreads();
-  if (tid < TQ && cnt_sh[tid] && q0 + tid < a.Q) atomicAdd(&a.counts[q0 + tid], cnt_sh[tid]);
 }
 
 // exact canonical re-score of a list of ambiguous (query, entity) pairs (tcgen05 path, kge_eval_gemm.cu)
@@ -168,10 +217,50 @@ __global__ void rescore_pairs_kernel(const int2 *__restrict__ amb, const int *__
   }
 }
 
+// The same for the stats kernels: each pair (never the positive's column) is classified by the filter bitmap and
+// settled as greater / equal before / equal after the positive; stats is [Q, KGE_RANK_STATS].
+template <int OP>
+__global__ void rescore_pair_stats_kernel(const int2 *__restrict__ amb, const int *__restrict__ amb_count, int capacity,
+                                          const float *__restrict__ qvec, const float *__restrict__ E, int d, int De,
+                                          const float *__restrict__ pos_score, const int64_t *__restrict__ queries,
+                                          int pos_col, float gamma, const float *__restrict__ modulus,
+                                          const uint32_t *__restrict__ filter_bits, int words,
+                                          int32_t *__restrict__ stats) {
+  int n = amb_count[0];
+  if (n > capacity) n = capacity;
+  const int lane = threadIdx.x & 31;
+  const int wid = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, nw = (gridDim.x * blockDim.x) >> 5;
+  for (int i = wid; i < n; i += nw) {
+    const int2 p = amb[i];
+    const float s = finish_exact<OP>(canonical_pair_score<OP>(qvec + (int64_t)p.x * De, E + (int64_t)p.y * De, d),
+                                     gamma, modulus ? modulus[0] : 1.f);
+    if (lane == 0) {
+      const float sp = pos_score[p.x];
+      const int64_t pid = queries[(int64_t)p.x * 3 + pos_col];
+      const int k = s > sp ? 0 : s == sp ? (p.y < pid ? 1 : 2) : -1;
+      if (k >= 0) {
+        int32_t *row = stats + (int64_t)p.x * KGE_RANK_STATS;
+        if (!((filter_bits[(int64_t)p.x * words + (p.y >> 5)] >> (p.y & 31)) & 1u)) atomicAdd(row + k, 1);
+        atomicAdd(row + k + 3, 1);
+      }
+    }
+  }
+}
+
+// filter_bits non-null: the stats re-score (counts is then [Q, KGE_RANK_STATS])
 int launch_rescore_pairs(bool cplx, const void *amb, const int *amb_count, int capacity, const float *qvec,
                          const float *E, int d, int De, const float *pos_score, const int64_t *queries, int pos_col,
-                         int32_t *counts, cudaStream_t st) {
-  if (cplx)
+                         int32_t *counts, cudaStream_t st, const uint32_t *filter_bits, int words) {
+  if (filter_bits) {
+    if (cplx)
+      rescore_pair_stats_kernel<OP_CMUL><<<148 * 8, 256, 0, st>>>((const int2 *)amb, amb_count, capacity, qvec, E, d, De,
+                                                                  pos_score, queries, pos_col, 0.f, nullptr,
+                                                                  filter_bits, words, counts);
+    else
+      rescore_pair_stats_kernel<OP_MUL><<<148 * 8, 256, 0, st>>>((const int2 *)amb, amb_count, capacity, qvec, E, d, De,
+                                                                 pos_score, queries, pos_col, 0.f, nullptr,
+                                                                 filter_bits, words, counts);
+  } else if (cplx)
     rescore_pairs_kernel<OP_CMUL><<<148 * 8, 256, 0, st>>>((const int2 *)amb, amb_count, capacity, qvec, E, d, De,
                                                            pos_score, queries, pos_col, 0.f, counts);
   else
@@ -263,7 +352,7 @@ __global__ void filter_lookup_dense_kernel(const int32_t *__restrict__ offsets, 
   }
 }
 
-template <int OP>
+template <int OP, bool STATS>
 static int launch_count(const EvalArgs &a, bool aligned, cudaStream_t st) {
   constexpr int H = op_is_complex(OP) ? 2 : 1;
   const size_t smem = sizeof(float) * 2 * (TQ + TJ) * H * ST;
@@ -271,22 +360,27 @@ static int launch_count(const EvalArgs &a, bool aligned, cudaStream_t st) {
   if constexpr (OP == OP_CDIST || OP == OP_SUBSIN || OP == OP_ADDSIN) {
     if (a.amb && aligned && a.d <= kFastMaxD) {                      // two-stage: fast tile pass + exact re-score
       KGE_CUDA_OK(cudaMemsetAsync(a.amb_count, 0, 2 * sizeof(int), st));
-      auto k = count_ranks_kernel<OP, true, true>;
+      auto k = count_ranks_kernel<OP, true, true, STATS>;
       KGE_CUDA_OK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
       k<<<grid, EVAL_THREADS, smem, st>>>(a);
       KGE_CUDA_OK(cudaGetLastError());
-      rescore_pairs_kernel<OP><<<148 * 4, 256, 0, st>>>(a.amb, a.amb_count, a.amb_capacity, a.qvec, a.X, a.d, a.De,
-                                                        a.pos_score, a.queries, a.pos_col, a.gamma, a.counts, a.modulus);
+      if constexpr (STATS)
+        rescore_pair_stats_kernel<OP><<<148 * 4, 256, 0, st>>>(a.amb, a.amb_count, a.amb_capacity, a.qvec, a.X, a.d,
+                                                               a.De, a.pos_score, a.queries, a.pos_col, a.gamma,
+                                                               a.modulus, a.filter_bits, a.words, a.counts);
+      else
+        rescore_pairs_kernel<OP><<<148 * 4, 256, 0, st>>>(a.amb, a.amb_count, a.amb_capacity, a.qvec, a.X, a.d, a.De,
+                                                          a.pos_score, a.queries, a.pos_col, a.gamma, a.counts, a.modulus);
       KGE_CUDA_OK(cudaGetLastError());
       return KGE_OK;
     }
   }
   if (aligned) {
-    auto k = count_ranks_kernel<OP, true>;
+    auto k = count_ranks_kernel<OP, true, false, STATS>;
     KGE_CUDA_OK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     k<<<grid, EVAL_THREADS, smem, st>>>(a);
   } else {
-    auto k = count_ranks_kernel<OP, false>;
+    auto k = count_ranks_kernel<OP, false, false, STATS>;
     KGE_CUDA_OK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     k<<<grid, EVAL_THREADS, smem, st>>>(a);
   }
@@ -379,7 +473,7 @@ extern "C" int kge_eval_positive_scores(const kge_model_t *m, int mode, const fl
 static int count_ranks_impl(const kge_model_t *m, int mode, const float *qvec, const int64_t *queries, int64_t Q,
                             const float *phase_table, const float *pos_score, const uint32_t *filter_bits,
                             int64_t ent_begin, int64_t ent_end, int32_t *counts, float *scores_out, void *amb_pairs,
-                            int64_t amb_capacity, int32_t *amb_count, void *stream);
+                            int64_t amb_capacity, int32_t *amb_count, void *stream, bool stats = false);
 
 extern "C" int kge_eval_count_ranks(const kge_model_t *m, int mode, const float *qvec, const int64_t *queries, int64_t Q,
                                     const float *phase_table, const float *pos_score, const uint32_t *filter_bits,
@@ -410,6 +504,24 @@ extern "C" int kge_eval_count_ranks_two_stage_approx(const kge_model_t *m, int m
                           approx_scores_out, amb_pairs, amb_capacity, amb_count, stream);
 }
 
+extern "C" int kge_eval_count_rank_stats(const kge_model_t *m, int mode, const float *qvec, const int64_t *queries,
+                                         int64_t Q, const float *phase_table, const float *pos_score,
+                                         const uint32_t *filter_bits, int64_t ent_begin, int64_t ent_end, int32_t *stats,
+                                         void *stream) {
+  return count_ranks_impl(m, mode, qvec, queries, Q, phase_table, pos_score, filter_bits, ent_begin, ent_end, stats,
+                          nullptr, nullptr, 0, nullptr, stream, true);
+}
+
+extern "C" int kge_eval_count_rank_stats_two_stage(const kge_model_t *m, int mode, const float *qvec,
+                                                   const int64_t *queries, int64_t Q, const float *phase_table,
+                                                   const float *pos_score, const uint32_t *filter_bits,
+                                                   int64_t ent_begin, int64_t ent_end, int32_t *stats, void *amb_pairs,
+                                                   int64_t amb_capacity, int32_t *amb_count, void *stream) {
+  KGE_REQUIRE(amb_pairs && amb_count && amb_capacity > 0, "two-stage ranking needs the ambiguous-pair buffers");
+  return count_ranks_impl(m, mode, qvec, queries, Q, phase_table, pos_score, filter_bits, ent_begin, ent_end, stats,
+                          nullptr, amb_pairs, amb_capacity, amb_count, stream, true);
+}
+
 extern "C" int kge_eval_two_stage_band(int model, int64_t entity_dim, float modulus, float *host_band) {
   KGE_REQUIRE(host_band, "null pointer");
   KGE_REQUIRE(model == KGE_ROTATE || model == KGE_PROTATE, "model %d has no two-stage pass", model);
@@ -426,7 +538,7 @@ extern "C" int kge_eval_two_stage_band(int model, int64_t entity_dim, float modu
 static int count_ranks_impl(const kge_model_t *m, int mode, const float *qvec, const int64_t *queries, int64_t Q,
                             const float *phase_table, const float *pos_score, const uint32_t *filter_bits,
                             int64_t ent_begin, int64_t ent_end, int32_t *counts, float *scores_out, void *amb_pairs,
-                            int64_t amb_capacity, int32_t *amb_count, void *stream) {
+                            int64_t amb_capacity, int32_t *amb_count, void *stream, bool stats) {
   int rc = check_model(m);
   if (rc) return rc;
   bool head;
@@ -447,7 +559,7 @@ static int count_ranks_impl(const kge_model_t *m, int mode, const float *qvec, c
   cudaStream_t st = (cudaStream_t)stream;
 #define KGE_CR(OP) \
   case OP:         \
-    return launch_count<OP>(a, aligned, st);
+    return stats ? launch_count<OP, true>(a, aligned, st) : launch_count<OP, false>(a, aligned, st);
   switch (op_of(m->model, head)) {
     KGE_CR(OP_SUBABS) KGE_CR(OP_ADDABS) KGE_CR(OP_MUL) KGE_CR(OP_CMUL) KGE_CR(OP_CDIST) KGE_CR(OP_SUBSIN)
     KGE_CR(OP_ADDSIN)

@@ -117,6 +117,9 @@ __host__ __device__ constexpr uint32_t instr_desc_tf32(int M, int N) {
   return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
 
+// STATS: a.counts is the [Q, KGE_RANK_STATS] table of kge_eval_gemm_count_rank_stats; filtered columns are classified too
+// (their approximation against the band), and the kernel adds counters [0] (unfiltered, greater) and [3] (greater).
+template <bool STATS>
 __global__ void __launch_bounds__(GTHREADS, 1)
 gemm_count_kernel(const __grid_constant__ CUtensorMap tmQhi, const __grid_constant__ CUtensorMap tmQlo,
                   const __grid_constant__ CUtensorMap tmEhi, const __grid_constant__ CUtensorMap tmElo,
@@ -216,6 +219,7 @@ gemm_count_kernel(const __grid_constant__ CUtensorMap tmQhi, const __grid_consta
     const int64_t pid = qvalid ? a.queries[(int64_t)qi * 3 + a.pos_col] : -1;
     const uint32_t *frow = a.filter_bits + (int64_t)(qvalid ? qi : 0) * a.words;
     int count = 0;
+    [[maybe_unused]] int count_raw = 0;
     int tile_it = 0;
     for (int64_t jt = blockIdx.y; jt < ntiles_all; jt += gridDim.y, ++tile_it) {
       const int as = tile_it & 1;
@@ -252,11 +256,17 @@ gemm_count_kernel(const __grid_constant__ CUtensorMap tmQhi, const __grid_consta
           for (int i = 0; i < 32; ++i) {
             const int64_t j = jb + i;
             if (a.approx_out && j < a.ent_end) a.approx_out[(int64_t)qi * a.nentity + j] = __uint_as_float(v[i]);
-            if (j >= a.ent_end || j == pid || ((fw >> i) & 1u)) continue;
+            if (j >= a.ent_end || j == pid || (!STATS && ((fw >> i) & 1u))) continue;
             const float s = __uint_as_float(v[i]);
             const float eps = qn * enorm_s[as * GN + c * 32 + i];
-            if (s - eps > sp) ++count;
-            else if (s + eps >= sp) am |= 1u << i;             // cannot be decided from the approximation
+            if (s - eps > sp) {
+              if constexpr (STATS) {
+                count += !((fw >> i) & 1u);
+                ++count_raw;
+              } else {
+                ++count;
+              }
+            } else if (s + eps >= sp) am |= 1u << i;           // cannot be decided from the approximation
           }
         }
         amask[c] = am;
@@ -292,7 +302,12 @@ gemm_count_kernel(const __grid_constant__ CUtensorMap tmQhi, const __grid_consta
         }
       }
     }
-    if (qvalid && count) atomicAdd(a.counts + qi, count);
+    if constexpr (STATS) {
+      if (qvalid && count) atomicAdd(a.counts + (int64_t)qi * KGE_RANK_STATS, count);
+      if (qvalid && count_raw) atomicAdd(a.counts + (int64_t)qi * KGE_RANK_STATS + 3, count_raw);
+    } else {
+      if (qvalid && count) atomicAdd(a.counts + qi, count);
+    }
   }
 
   tc_fence_before();
@@ -332,7 +347,8 @@ __global__ void split_tf32_kernel(const float *__restrict__ x, int64_t rows, int
 
 int launch_rescore_pairs(bool cplx, const void *amb, const int *amb_count, int capacity, const float *qvec,
                          const float *E, int d, int De, const float *pos_score, const int64_t *queries, int pos_col,
-                         int32_t *counts, cudaStream_t st);                       // kge_eval.cu (exact op sequence)
+                         int32_t *counts, cudaStream_t st, const uint32_t *filter_bits = nullptr,
+                         int words = 0);                                          // kge_eval.cu (exact op sequence)
 
 // ---- host ---------------------------------------------------------------------------------------------------
 typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
@@ -382,12 +398,11 @@ extern "C" int kge_eval_gemm_split(const float *x, int64_t rows, int64_t cols, f
   return KGE_OK;
 }
 
-extern "C" int kge_eval_gemm_count_ranks(const kge_model_t *m, int mode, const float *qvec, const float *qhi,
-                                         const float *qlo, const float *qnorm, const int64_t *queries, int64_t Q,
-                                         const float *pos_score, const uint32_t *filter_bits, const float *ehi,
-                                         const float *elo, const float *enorm, int64_t ent_begin, int64_t ent_end,
-                                         int32_t *counts, void *amb_pairs, int64_t amb_capacity, int32_t *amb_count,
-                                         float *approx_scores_out, void *stream) {
+static int gemm_count_impl(const kge_model_t *m, int mode, const float *qvec, const float *qhi, const float *qlo,
+                           const float *qnorm, const int64_t *queries, int64_t Q, const float *pos_score,
+                           const uint32_t *filter_bits, const float *ehi, const float *elo, const float *enorm,
+                           int64_t ent_begin, int64_t ent_end, int32_t *counts, void *amb_pairs, int64_t amb_capacity,
+                           int32_t *amb_count, float *approx_scores_out, void *stream, bool stats) {
   int rc = check_model(m);
   if (rc) return rc;
   KGE_REQUIRE(kge_eval_gemm_supported(m), "the tcgen05 path serves DistMult / ComplEx with 16-byte aligned rows");
@@ -416,18 +431,39 @@ extern "C" int kge_eval_gemm_count_ranks(const kge_model_t *m, int mode, const f
   a.approx_out = approx_scores_out;
   KGE_CUDA_OK(cudaMemsetAsync(amb_count, 0, 2 * sizeof(int), st));
   const size_t smem = GSTAGES * kStageBytes + (2 * GSTAGES + 4) * 8 + 16 + 2 * GN * 4 + 1024;
-  KGE_CUDA_OK(cudaFuncSetAttribute(gemm_count_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  auto kernel = stats ? gemm_count_kernel<true> : gemm_count_kernel<false>;
+  KGE_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int qtiles = (int)((Q + GM - 1) / GM);
   const int64_t jtiles = (ent_end - ent_begin + GN - 1) / GN;
   int ysplit = 148 / qtiles;                                      // one wave: at most 148 CTAs (one per SM)
   if (ysplit > jtiles) ysplit = (int)jtiles;
   if (ysplit < 1) ysplit = 1;
-  gemm_count_kernel<<<dim3(qtiles, ysplit), GTHREADS, smem, st>>>(tQhi, tQlo, tEhi, tElo, a);
+  kernel<<<dim3(qtiles, ysplit), GTHREADS, smem, st>>>(tQhi, tQlo, tEhi, tElo, a);
   KGE_CUDA_OK(cudaGetLastError());
   const bool cplx = m->model == KGE_COMPLEX;
   const int d = cplx ? (int)(K / 2) : (int)K;
   if ((rc = launch_rescore_pairs(cplx, a.amb, amb_count, a.amb_capacity, qvec, m->entity, d, (int)K, pos_score, queries,
-                                 a.pos_col, counts, st)))
+                                 a.pos_col, counts, st, stats ? filter_bits : nullptr, a.words)))
     return rc;
   return KGE_OK;
+}
+
+extern "C" int kge_eval_gemm_count_ranks(const kge_model_t *m, int mode, const float *qvec, const float *qhi,
+                                         const float *qlo, const float *qnorm, const int64_t *queries, int64_t Q,
+                                         const float *pos_score, const uint32_t *filter_bits, const float *ehi,
+                                         const float *elo, const float *enorm, int64_t ent_begin, int64_t ent_end,
+                                         int32_t *counts, void *amb_pairs, int64_t amb_capacity, int32_t *amb_count,
+                                         float *approx_scores_out, void *stream) {
+  return gemm_count_impl(m, mode, qvec, qhi, qlo, qnorm, queries, Q, pos_score, filter_bits, ehi, elo, enorm, ent_begin,
+                         ent_end, counts, amb_pairs, amb_capacity, amb_count, approx_scores_out, stream, false);
+}
+
+extern "C" int kge_eval_gemm_count_rank_stats(const kge_model_t *m, int mode, const float *qvec, const float *qhi,
+                                              const float *qlo, const float *qnorm, const int64_t *queries, int64_t Q,
+                                              const float *pos_score, const uint32_t *filter_bits, const float *ehi,
+                                              const float *elo, const float *enorm, int64_t ent_begin, int64_t ent_end,
+                                              int32_t *stats, void *amb_pairs, int64_t amb_capacity,
+                                              int32_t *amb_count, void *stream) {
+  return gemm_count_impl(m, mode, qvec, qhi, qlo, qnorm, queries, Q, pos_score, filter_bits, ehi, elo, enorm, ent_begin,
+                         ent_end, stats, amb_pairs, amb_capacity, amb_count, nullptr, stream, true);
 }

@@ -924,6 +924,34 @@ class KGEModel(nn.Module):
         """Filtered rank of every test triple in `mode` (model.py:382-418 without the sort): int64 [len].
         Entities are sharded across the ranks of an initialised process group; the integer counts are
         all-reduced (bit-exact)."""
+        counts, scores, approx = self._entity_rank_counts(test_triples, all_true_triples, mode, query_chunk, exact,
+                                                          False, return_scores, return_approx)
+        ranks = counts + 1
+        if return_approx:
+            return ranks, approx
+        return (ranks, scores) if return_scores else ranks
+
+    RANK_STATS = 6          # KGE_RANK_STATS of include/kge_b200.h
+
+    def rank_statistics(self, test_triples, all_true_triples, mode, query_chunk=4096, exact=False):
+        """Raw and tie-aware rank statistics of every test triple in `mode`: int64 numpy [len, 6], per query the number
+        of candidate entities j != the positive with
+          [0] j not filtered, s_j > s_pos          [3] s_j > s_pos
+          [1] j not filtered, s_j == s_pos, j < pos  [4] s_j == s_pos, j < pos
+          [2] j not filtered, s_j == s_pos, j > pos  [5] s_j == s_pos, j > pos
+        where j is filtered when it completes the query into a triple of all_true_triples and s is the exact score of
+        filtered_ranks (NaN is never greater or equal, -0.0 == +0.0).  1 + [0] + [1] is filtered_ranks' rank (for
+        |s_pos| < 2^24, where its filter bias s_pos - 1 stays below s_pos) and
+        1 + [3] + [4] the raw rank; ranks_from_statistics turns the table into optimistic, pessimistic or realistic
+        ranks.  The path is filtered_ranks' (exact=True or KGE_EVAL_SIMT=1: the exact tile kernel); with an initialised
+        process group every rank counts over its entity slice and the tallies are all-reduced (a collective: call it on
+        every rank)."""
+        return self._entity_rank_counts(test_triples, all_true_triples, mode, query_chunk, exact, True)[0]
+
+    def _entity_rank_counts(self, test_triples, all_true_triples, mode, query_chunk, exact, stats,
+                            return_scores=False, return_approx=False):
+        """The query loop of filtered_ranks (stats=False: int64 counts [len]) and rank_statistics (stats=True: int64
+        [len, 6]), with the [len, nentity] score dumps of filtered_ranks (None when not asked for)."""
         dev = self._device()
         st = _stream(dev)
         nentity, nrelation = self.entity_embedding.shape[0], self.relation_embedding.shape[0]
@@ -957,8 +985,9 @@ class KGEModel(nn.Module):
         # one int32 buffer [rank counts | per-chunk (ambiguous pairs, overflow flag)]: a single all-reduce and a single
         # read-back per call
         nq_all = queries_all.shape[0]
-        tally = torch.zeros(nq_all + 2 * max(nchunks, 1), dtype=torch.int32, device=dev)
-        amb_counts = tally[nq_all:].view(-1, 2) if (gemm or two_stage) else None
+        ncol = self.RANK_STATS if stats else 1
+        tally = torch.zeros(nq_all * ncol + 2 * max(nchunks, 1), dtype=torch.int32, device=dev)
+        amb_counts = tally[nq_all * ncol:].view(-1, 2) if (gemm or two_stage) else None
         if gemm:
             nE = self.entity_embedding.numel()
             ehi = self._buffer('gemm_ehi', nE, torch.float32, dev)
@@ -966,7 +995,7 @@ class KGEModel(nn.Module):
             enorm = self._buffer('gemm_enorm', nentity, torch.float32, dev)
             _lib.call("kge_eval_gemm_split", _ptr(self.entity_embedding), nentity, self.entity_dim, _ptr(ehi), _ptr(elo),
                       _ptr(enorm), st)
-        counts_all = tally[:nq_all]
+        counts_all = tally[:nq_all * ncol]
         scores = torch.empty((queries_all.shape[0], nentity), dtype=torch.float32, device=dev) if return_scores else None
         # tests: the approximations of the tcgen05 path or of the two-stage fast pass (to pin their error bands against
         # exact scores)
@@ -979,7 +1008,7 @@ class KGEModel(nn.Module):
             bits = self._buffer('filter_bits', Q * words, torch.int32, dev)
             qvec = self._buffer('qvec', Q * self.entity_dim, torch.float32, dev)
             pos = self._buffer('pos_score', Q, torch.float32, dev)
-            counts = counts_all[lo:lo + Q]
+            counts = counts_all[lo * ncol:(lo + Q) * ncol]
             # filter bitmap of the chunk, looked up on the device in the resident index (dataloader.py:134-154)
             if ftab[0] == 'dense':
                 _lib.call("kge_eval_filter_bits_lookup_dense", _ptr(ftab[1]), _ptr(ftab[2]), _ptr(queries), Q, m, nentity,
@@ -1001,20 +1030,32 @@ class KGEModel(nn.Module):
                 cap = int(os.environ.get('KGE_EVAL_AMB_CAP', Q * 1024))
                 amb = self._buffer('gemm_amb', cap * 2, torch.int32, dev)
                 _lib.call("kge_eval_gemm_split", _ptr(qvec), Q, self.entity_dim, _ptr(qhi), _ptr(qlo), _ptr(qnorm), st)
-                _lib.call("kge_eval_gemm_count_ranks", ctypes.byref(desc), m, _ptr(qvec), _ptr(qhi), _ptr(qlo),
-                          _ptr(qnorm), _ptr(queries), Q, _ptr(pos), _ptr(bits), _ptr(ehi), _ptr(elo), _ptr(enorm),
-                          ent_begin, ent_end, _ptr(counts), _ptr(amb), cap, _ptr(amb_counts[ci]),
-                          _ptr(approx[lo:lo + Q]) if approx is not None else None, st)
+                gemm_args = (ctypes.byref(desc), m, _ptr(qvec), _ptr(qhi), _ptr(qlo), _ptr(qnorm), _ptr(queries), Q,
+                             _ptr(pos), _ptr(bits), _ptr(ehi), _ptr(elo), _ptr(enorm), ent_begin, ent_end, _ptr(counts),
+                             _ptr(amb), cap, _ptr(amb_counts[ci]))
+                if stats:
+                    _lib.call("kge_eval_gemm_count_rank_stats", *gemm_args, st)
+                else:
+                    _lib.call("kge_eval_gemm_count_ranks", *gemm_args,
+                              _ptr(approx[lo:lo + Q]) if approx is not None else None, st)
             elif two_stage:
                 cap = int(os.environ.get('KGE_EVAL_AMB_CAP', Q * 256))
                 amb = self._buffer('gemm_amb', cap * 2, torch.int32, dev)
-                _lib.call("kge_eval_count_ranks_two_stage_approx", ctypes.byref(desc), m, _ptr(qvec), _ptr(queries), Q,
-                          _ptr(phase), _ptr(pos), _ptr(bits), ent_begin, ent_end, _ptr(counts), _ptr(amb), cap,
-                          _ptr(amb_counts[ci]), _ptr(approx[lo:lo + Q]) if approx is not None else None, st)
+                two_stage_args = (ctypes.byref(desc), m, _ptr(qvec), _ptr(queries), Q, _ptr(phase), _ptr(pos), _ptr(bits),
+                                  ent_begin, ent_end, _ptr(counts), _ptr(amb), cap, _ptr(amb_counts[ci]))
+                if stats:
+                    _lib.call("kge_eval_count_rank_stats_two_stage", *two_stage_args, st)
+                else:
+                    _lib.call("kge_eval_count_ranks_two_stage_approx", *two_stage_args,
+                              _ptr(approx[lo:lo + Q]) if approx is not None else None, st)
             else:
-                _lib.call("kge_eval_count_ranks", ctypes.byref(desc), m, _ptr(qvec), _ptr(queries), Q, _ptr(phase),
-                          _ptr(pos), _ptr(bits), ent_begin, ent_end, _ptr(counts),
-                          _ptr(scores[lo:lo + Q]) if scores is not None else None, st)
+                exact_args = (ctypes.byref(desc), m, _ptr(qvec), _ptr(queries), Q, _ptr(phase), _ptr(pos), _ptr(bits),
+                              ent_begin, ent_end, _ptr(counts))
+                if stats:
+                    _lib.call("kge_eval_count_rank_stats", *exact_args, st)
+                else:
+                    _lib.call("kge_eval_count_ranks", *exact_args,
+                              _ptr(scores[lo:lo + Q]) if scores is not None else None, st)
             if events is not None:
                 ev1.record()
                 events.append((ev0, ev1))
@@ -1022,18 +1063,19 @@ class KGEModel(nn.Module):
             torch.distributed.all_reduce(tally)              # integer sums over the entity shards: bit-exact; an
             #                                                  overflow flag on any rank re-runs the chunk everywhere
         host = tally.cpu().numpy()                           # the call's one host sync
-        ranks = host[:nq_all].astype(np.int64) + 1
+        counts = host[:nq_all * ncol].astype(np.int64)
+        if stats:
+            counts = counts.reshape(nq_all, ncol)
         if amb_counts is not None:
-            stats = host[nq_all:].reshape(-1, 2)
-            self._ws['gemm_last_ambiguous' if gemm else 'two_stage_last_ambiguous'] = int(stats[:, 0].sum())
-            for ci in np.nonzero(stats[:, 1])[0]:            # ambiguous list overflowed: exact kernel for that chunk
+            amb_host = host[nq_all * ncol:].reshape(-1, 2)
+            self._ws['gemm_last_ambiguous' if gemm else 'two_stage_last_ambiguous'] = int(amb_host[:, 0].sum())
+            for ci in np.nonzero(amb_host[:, 1])[0]:         # ambiguous list overflowed: exact kernel for that chunk
                 lo = int(ci) * query_chunk
                 chunk = [tuple(int(v) for v in row) for row in queries_all[lo:lo + query_chunk]]
-                ranks[lo:lo + query_chunk] = self.filtered_ranks(chunk, all_true_triples, mode, query_chunk, exact=True)
+                counts[lo:lo + query_chunk] = self._entity_rank_counts(chunk, all_true_triples, mode, query_chunk, True,
+                                                                       stats)[0]
         self._raise_if_bad_index()
-        if return_approx:
-            return ranks, approx
-        return (ranks, scores) if return_scores else ranks
+        return counts, scores, approx
 
     TOPK_MAX = 256          # KGE_TOPK_MAX of include/kge_b200.h
 
@@ -1319,6 +1361,31 @@ class KGEModel(nn.Module):
                         logging.info('Evaluating the model... (%d/%d)' % (step, total_steps))
                     step += 1
         return metrics_from_ranks(np.concatenate(all_ranks))
+
+
+def ranks_from_statistics(stats, filtered=True, ties='stable'):
+    """Ranks from the [len, 6] table of KGEModel.rank_statistics: the filtered (filtered=True) or raw ranks, with the
+    positive placed among the candidates of equal score
+      'optimistic'   first:              1 + greater
+      'stable'       by entity id:       1 + greater + equal_before        (filtered: the rank of filtered_ranks)
+      'pessimistic'  last:               1 + greater + equal_before + equal_after
+      'realistic'    in the middle:      1 + greater + (equal_before + equal_after) / 2   (the expected rank under a random
+                                         order of the ties)
+    int64 [len], float64 for 'realistic'; metrics_from_ranks turns them into MRR / MR / HITS@k."""
+    table = np.asarray(stats)
+    if table.ndim != 2 or table.shape[1] != KGEModel.RANK_STATS or not np.issubdtype(table.dtype, np.integer):
+        raise ValueError('stats must be an integer table [len, %d] (KGEModel.rank_statistics), got %s %s'
+                         % (KGEModel.RANK_STATS, table.dtype, table.shape))
+    g, eb, ea = (table[:, c].astype(np.int64) for c in ((0, 1, 2) if filtered else (3, 4, 5)))
+    if ties == 'optimistic':
+        return 1 + g
+    if ties == 'stable':
+        return 1 + g + eb
+    if ties == 'pessimistic':
+        return 1 + g + eb + ea
+    if ties == 'realistic':
+        return 1.0 + g + (eb + ea) / 2.0
+    raise ValueError("ties must be 'optimistic', 'stable', 'pessimistic' or 'realistic', got %r" % (ties,))
 
 
 def metrics_from_ranks(ranks):
