@@ -281,6 +281,21 @@ int kge_eval_gemm_count_rank_stats(const kge_model_t *m, int mode, const float *
                                    int32_t *stats, void *amb_pairs, int64_t amb_capacity, int32_t *amb_count,
                                    void *stream);
 
+/* ---- candidate-list ranking: each query against its own list of entities (sampled evaluation, OGB-style) ----
+ * candidates [Q, ld] int64 entity ids of the predicted slot; -1 is padding (anywhere in a row); any other id outside
+ * [0, nentity) sets *err_flag and counts nothing.  For the listed entries j in columns [col_begin, col_end) with
+ * j != pos(q), counted as often as they are listed, stats [Q, KGE_RANK_STATS] (zeroed by the caller) receives the
+ * counters of kge_eval_count_rank_stats, "filtered" read from filter_bits ([Q, ceil(nentity/32)], or NULL: nothing is
+ * filtered).  s is the canonical score of kge_eval_count_ranks (bit-identical).  qvec and pos_score come from
+ * kge_eval_query_vectors and kge_eval_positive_scores; pRotatE also needs kge_eval_phase_table.  The counters add up
+ * over column slices.  scores_out [Q, ld] (may be NULL) receives the scores of the slice's columns: s for a listed
+ * entity, s_pos where it names the positive, -inf at padding.  At most 65535*128 columns per slice.                 */
+int kge_eval_candidate_rank_stats(const kge_model_t *m, int mode, const float *qvec, const int64_t *queries,
+                                  int64_t Q, const float *phase_table, const float *pos_score,
+                                  const int64_t *candidates, int64_t ld, int64_t col_begin, int64_t col_end,
+                                  const uint32_t *filter_bits, int32_t *stats, float *scores_out, int32_t *err_flag,
+                                  void *stream);
+
 /* filter bitmap from a CSR of true entities per query (dataloader.py:138-144)                     */
 int kge_eval_filter_bits(const int64_t *csr_offsets, const int32_t *csr_entities, int64_t Q,
                          int64_t nentity, uint32_t *filter_bits, void *stream);

@@ -44,6 +44,13 @@ def _on_device(t, dev, dtype, stage=None, st=None):
     return t.to(device=dev, dtype=dtype, non_blocking=True).contiguous()
 
 
+def _is_integer(a):
+    """An integer (not bool) numpy array or torch tensor."""
+    if isinstance(a, torch.Tensor):
+        return not a.dtype.is_floating_point and not a.dtype.is_complex and a.dtype != torch.bool
+    return np.issubdtype(a.dtype, np.integer)
+
+
 def _dist():
     """(rank, world_size) of the data-parallel group, (0, 1) when torch.distributed is not initialised."""
     import torch.distributed as dist
@@ -1076,6 +1083,118 @@ class KGEModel(nn.Module):
                                                                        stats)[0]
         self._raise_if_bad_index()
         return counts, scores, approx
+
+    # device bytes of the exclusion bitmap of one query chunk (nentity / 8 per query): at 2.5 M entities a 4096-query
+    # chunk would need 1.3 GB, so candidate_rank_statistics shrinks its chunk to stay within this
+    _CAND_BITS_BUDGET = 1 << 28
+
+    def candidate_rank_statistics(self, queries, candidates, mode, exclude_triples=None, query_chunk=4096,
+                                  return_scores=False):
+        """Rank statistics of every query against its own list of candidate entities (sampled evaluation, as in OGB's
+        ogbl-wikikg2 / ogbl-biokg evaluators): int64 numpy [Q, 6] with the columns of rank_statistics, counted over the
+        listed entries instead of all entities.
+
+        queries: (h, r, t) tuples or an int64 array / tensor [Q, 3] (the layout of test_triples); the positive is the
+        entity in the predicted slot ('head-batch': h, 'tail-batch': t).  candidates: int64 array / tensor [Q, C] (any
+        device) or a list of equal-length lists of entity ids for the predicted slot; -1 is padding and may appear
+        anywhere in a row, so ragged lists work.  Any other id outside [0, nentity) raises IndexError.  Per query, over
+        the listed entries j (counted as often as they are listed; an entry naming the positive itself is skipped):
+          [0] j not excluded, s_j > s_pos          [3] s_j > s_pos
+          [1] j not excluded, s_j == s_pos, j < pos  [4] s_j == s_pos, j < pos
+          [2] j not excluded, s_j == s_pos, j > pos  [5] s_j == s_pos, j > pos
+        where j is excluded when it completes the query into a triple of exclude_triples (the filter of filtered_ranks)
+        and s is the canonical exact score of filtered_ranks (NaN is never greater or equal, -0.0 == +0.0).
+        ranks_from_statistics and metrics_from_ranks take the table unchanged; ranks_from_statistics(stats,
+        filtered=False, ties='realistic') is OGB's rank 1 + #{neg > pos} + #{neg == pos} / 2, with two differences from
+        OGB's evaluator: a negative that names the positive counts as a tie there and is skipped here, and OGB's scores
+        come from torch, so near-ties may order differently.
+
+        return_scores: also a float32 tensor [Q, C] on the model's device with the canonical score of every listed entry
+        (s_pos, bit for bit, where an entry names the positive) and -inf at padding.  With an initialised process group
+        every rank counts its slice of the candidate columns and the tallies are all-reduced (a collective: call it on
+        every rank); return_scores then raises ValueError."""
+        if mode not in ('head-batch', 'tail-batch'):
+            raise ValueError('negative batch mode %s not supported' % mode)
+        if isinstance(query_chunk, bool) or int(query_chunk) != query_chunk or int(query_chunk) < 1:
+            raise ValueError('query_chunk must be a positive integer, got %r' % (query_chunk,))
+        q_in = queries.detach() if isinstance(queries, torch.Tensor) else np.asarray(queries)
+        if q_in.ndim != 2 or q_in.shape[1] != 3 or not _is_integer(q_in):
+            raise ValueError('queries must be (h, r, t) triples: an integer array [Q, 3], got %s %s'
+                             % (q_in.dtype, tuple(q_in.shape)))
+        if isinstance(candidates, torch.Tensor):
+            c_in = candidates.detach()
+        else:
+            try:
+                c_in = np.asarray(candidates)
+            except ValueError:                     # ragged nested lists
+                raise ValueError('candidates must be an integer array [Q, C] (pad short lists with -1)') from None
+        if c_in.ndim != 2 or c_in.shape[0] != q_in.shape[0] or not _is_integer(c_in):
+            raise ValueError('candidates must be an integer array [Q, C] (pad short lists with -1) with Q = %d, got '
+                             '%s %s' % (q_in.shape[0], c_in.dtype, tuple(c_in.shape)))
+        rank, world = _dist()
+        if return_scores and world > 1:
+            raise ValueError('return_scores is single-process only: each rank scores a slice of the candidate columns')
+        dev = self._device()
+        st = _stream(dev)
+        nq, ncand = int(c_in.shape[0]), int(c_in.shape[1])
+        stats = torch.zeros(max(nq * self.RANK_STATS, 1), dtype=torch.int32, device=dev)
+        scores = torch.empty((nq, ncand), dtype=torch.float32, device=dev) if return_scores else None
+        if nq == 0 or ncand == 0:
+            out = np.zeros((nq, self.RANK_STATS), dtype=np.int64)
+            return (out, scores) if return_scores else out
+        queries_dev = torch.as_tensor(q_in).to(device=dev, dtype=torch.int64, non_blocking=True).contiguous()
+        cand_dev = torch.as_tensor(c_in).to(device=dev, dtype=torch.int64, non_blocking=True).contiguous()
+        nentity, nrelation = self.entity_embedding.shape[0], self.relation_embedding.shape[0]
+        words = (nentity + 31) // 32
+        ftab = None
+        chunk = int(query_chunk)
+        if exclude_triples is not None:
+            ftab = self._filter_tables(self._filter_index(exclude_triples, nentity, nrelation), mode, dev, st)
+            chunk = max(1, min(chunk, self._CAND_BITS_BUDGET // (4 * words)))
+        col_begin, col_end = shard_bounds(ncand, rank, world)
+        desc = self._descriptor()
+        err = self._err_flag()
+        phase = None
+        if self.model_name == 'pRotatE':
+            phase = self._buffer('phase_table', self.entity_embedding.numel(), torch.float32, dev)
+            _lib.call("kge_eval_phase_table", ctypes.byref(desc), _ptr(phase), st)
+        m = _lib.MODE_IDS[mode]
+        for lo in range(0, nq, chunk):
+            q = queries_dev[lo:lo + chunk]
+            Q = q.shape[0]
+            bits = None
+            if ftab is not None:
+                bits = self._buffer('cand_bits', Q * words, torch.int32, dev)
+                if ftab[0] == 'dense':
+                    _lib.call("kge_eval_filter_bits_lookup_dense", _ptr(ftab[1]), _ptr(ftab[2]), _ptr(q), Q, m, nentity,
+                              nrelation, _ptr(bits), st)
+                else:
+                    _lib.call("kge_eval_filter_bits_lookup", _ptr(ftab[1]), _ptr(ftab[2]), _ptr(ftab[3]), ftab[4],
+                              _ptr(q), Q, m, nentity, nrelation, _ptr(bits), st)
+            qvec = self._buffer('cand_qvec', Q * self.entity_dim, torch.float32, dev)
+            pos = self._buffer('cand_pos_score', Q, torch.float32, dev)
+            _lib.call("kge_eval_query_vectors", ctypes.byref(desc), m, _ptr(q), Q, _ptr(qvec), _ptr(err), st)
+            _lib.call("kge_eval_positive_scores", ctypes.byref(desc), m, _ptr(qvec), _ptr(q), Q, _ptr(phase), _ptr(pos),
+                      st)
+            events = self._ws.get('candidate_events')        # tools/candidate_rate.py: CUDA events around the kernel
+            if events is not None:
+                ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                ev0.record()
+            _lib.call("kge_eval_candidate_rank_stats", ctypes.byref(desc), m, _ptr(qvec), _ptr(q), Q, _ptr(phase),
+                      _ptr(pos), _ptr(cand_dev[lo:lo + Q]), ncand, col_begin, col_end, _ptr(bits),
+                      _ptr(stats[lo * self.RANK_STATS:(lo + Q) * self.RANK_STATS]),
+                      _ptr(scores[lo:lo + Q]) if scores is not None else None, _ptr(err), st)
+            if events is not None:
+                ev1.record()
+                events.append((ev0, ev1))
+        if world > 1:
+            import torch.distributed as dist
+            if dist.get_backend() == 'gloo':
+                stats = stats.cpu()
+            dist.all_reduce(stats)                           # integer sums over the column slices: bit-exact
+        out = stats.cpu().numpy()[:nq * self.RANK_STATS].astype(np.int64).reshape(nq, self.RANK_STATS)   # one host sync
+        self._raise_if_bad_index()
+        return (out, scores) if return_scores else out
 
     TOPK_MAX = 256          # KGE_TOPK_MAX of include/kge_b200.h
 
