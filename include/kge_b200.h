@@ -344,6 +344,33 @@ int kge_eval_topk(const kge_model_t *m, int mode, const float *qvec, int64_t Q, 
 int kge_eval_topk_merge(const uint64_t *keys_in, int64_t Q, int lists, int k, uint64_t *keys_out, int64_t *ids_out,
                         float *scores_out, void *stream);
 
+/* ---- similarity search: the k rows of the entity or relation table nearest to each query vector ----
+ * A row is the stored row as one flat real vector of the table's width (entity_dim / relation_dim; [re | im] together
+ * for double tables).  Scores are "larger is more similar", with acc() the canonical blocked sum of kge_eval_count_ranks
+ * (blocks of 32 summed in index order from +0.0f, block sums added in index order; correctly rounded, non-contracted):
+ *   KGE_SIM_DOT acc(q x)   KGE_SIM_COSINE acc(q x) / (|q| |x|)   KGE_SIM_L2 -sqrt(acc((q - x)^2))   KGE_SIM_L1 -acc(|q - x|)
+ * with |v| = sqrt(acc(v v)); a zero row under cosine gives 0/0 = NaN.  Order and key encoding are kge_eval_topk's.
+ * kge_similarity_rows: rows_out [Q, width] = the table rows ids [Q]; an id outside the table writes a zero row and sets
+ *   *err_flag (may be NULL).
+ * kge_similarity_norms: norms_out [n] = |v| of the table's rows (vectors == NULL, n must be the row count) or of n free
+ *   vectors [n, width].
+ * kge_similarity_topk: the k best rows in [row_begin, row_end) of each query vector qvec [Q, width], as keys_out [Q, k]
+ *   best first; cosine needs qnorm [Q] and xnorm [rows] from kge_similarity_norms.  self_ids [Q] (may be NULL): the row
+ *   left out of each query's list, -1 for none.  Merge the slices of several devices with kge_eval_topk_merge.  scratch:
+ *   kge_similarity_topk_scratch_bytes() (0 or more; a negative value is an error code).  At most 65535*64 queries per
+ *   call.                                                                                                          */
+enum { KGE_SIM_DOT = 0, KGE_SIM_COSINE = 1, KGE_SIM_L2 = 2, KGE_SIM_L1 = 3 };
+enum { KGE_TABLE_ENTITY = 0, KGE_TABLE_RELATION = 1 };
+int kge_similarity_rows(const kge_model_t *m, int table, const int64_t *ids, int64_t Q, float *rows_out,
+                        int32_t *err_flag, void *stream);
+int kge_similarity_norms(const kge_model_t *m, int table, const float *vectors, int64_t n, float *norms_out,
+                         void *stream);
+int64_t kge_similarity_topk_scratch_bytes(const kge_model_t *m, int table, int64_t Q, int64_t row_begin, int64_t row_end,
+                                          int k);
+int kge_similarity_topk(const kge_model_t *m, int table, int metric, const float *qvec, const float *qnorm,
+                        const float *xnorm, const int64_t *self_ids, int64_t Q, int64_t row_begin, int64_t row_end,
+                        int k, uint64_t *keys_out, void *scratch, int64_t scratch_bytes, void *stream);
+
 /* ---- relation prediction: which relation links h to t, for every query (h, ?, t) (queries [Q,3] int64, the relation
  *      slot is the positive for the ranks and is ignored by the top-k) ----
  * The score of relation r is the 'single'-mode score of (h, r, t) in the canonical order: bit-identical to column t of

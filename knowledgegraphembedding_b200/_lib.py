@@ -13,6 +13,8 @@ SINGLE, HEAD_BATCH, TAIL_BATCH = range(3)
 MODE_IDS = {"single": SINGLE, "head-batch": HEAD_BATCH, "tail-batch": TAIL_BATCH}
 LOSS_NEG_ADVERSARIAL, LOSS_NEG_UNIFORM, LOSS_POSITIVE = range(3)
 ERR_INVALID, ERR_CUDA, ERR_DEVICE = -1, -2, -3
+SIM_IDS = {"dot": 0, "cosine": 1, "l2": 2, "l1": 3}
+TABLE_ENTITY, TABLE_RELATION = range(2)
 
 
 class KgeModelStruct(Structure):
@@ -111,6 +113,11 @@ PROTOTYPES = {
     "kge_eval_topk": (c_int, [_M, c_int, c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_int64, c_int, c_void_p,
                               c_void_p, c_int64, c_void_p]),
     "kge_eval_topk_merge": (c_int, [c_void_p, c_int64, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "kge_similarity_rows": (c_int, [_M, c_int, c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),
+    "kge_similarity_norms": (c_int, [_M, c_int, c_void_p, c_int64, c_void_p, c_void_p]),
+    "kge_similarity_topk_scratch_bytes": (c_int64, [_M, c_int, c_int64, c_int64, c_int64, c_int]),
+    "kge_similarity_topk": (c_int, [_M, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64,
+                                    c_int, c_void_p, c_void_p, c_int64, c_void_p]),
     "kge_eval_relation_table": (c_int, [_M, c_void_p, c_void_p]),
     "kge_eval_relation_count_ranks": (c_int, [_M, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int64,
                                               c_int64, c_void_p, c_void_p, c_void_p]),

@@ -48,7 +48,8 @@ enum Op {
   OP_CMUL = 3,     // ComplEx:                  q_re x_re + q_im x_im
   OP_CDIST = 4,    // RotatE:                   |q - x| (complex modulus)
   OP_SUBSIN = 5,   // pRotatE tail/single:      |sin((ph+pr) - pt)|
-  OP_ADDSIN = 6    // pRotatE head-batch:       |sin(ph + (pr-pt))|
+  OP_ADDSIN = 6,   // pRotatE head-batch:       |sin(ph + (pr-pt))|
+  OP_SQDIFF = 7    // similarity search, l2:    (q - x)^2        (no model scores with it)
 };
 
 __host__ __device__ constexpr bool op_is_complex(int op) { return op == OP_CMUL || op == OP_CDIST; }

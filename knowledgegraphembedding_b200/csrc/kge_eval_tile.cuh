@@ -19,7 +19,11 @@ __device__ __forceinline__ float op_exact(float q0, float q1, float x0, float x1
     const float a = fsub(q0, x0), b = fsub(q1, x1);
     return fsqrt(ffma(b, b, fmul(a, a)));
   } else if constexpr (OP == OP_SUBSIN) return fabsf(sin_rep(fsub(q0, x0)));       // model.py:243-246 (x = phase table)
-  else return fabsf(sin_rep(fadd(x0, q0)));                                        // model.py:241
+  else if constexpr (OP == OP_ADDSIN) return fabsf(sin_rep(fadd(x0, q0)));         // model.py:241
+  else {                                                                           // similarity search, l2
+    const float t = fsub(q0, x0);
+    return fmul(t, t);
+  }
 }
 
 // Fast (non-canonical) element op of the two-stage RotatE evaluation: contraction allowed, one-instruction

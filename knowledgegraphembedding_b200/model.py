@@ -1442,6 +1442,111 @@ class KGEModel(nn.Module):
         self._raise_if_bad_index()                        # the call's one host sync
         return ids, scores
 
+    # ------------------------------------------------------------------------------------------ similarity search
+    def nearest_neighbors(self, items, table='entity', k=10, metric='cosine', exclude_self=True):
+        """Similarity search: the k rows of the entity or relation table closest to each query, best first.
+
+        table: 'entity' (rows of entity_embedding) or 'relation' (rows of relation_embedding).  A row is the stored row
+        as one flat real vector: [re | im] together for double tables, and the stored phases, unscaled, for RotatE /
+        pRotatE relations (phase wrap-around is not modelled).  items: 1-D integer row ids (list, array or tensor), or a
+        2-D float array / tensor [Q, width] of free query vectors (any device).  metric, "larger is more similar":
+        'dot' = acc(q x), 'cosine' = acc(q x) / (|q| |x|) with |v| = sqrt(acc(v v)), 'l2' = -sqrt(acc((q - x)^2)),
+        'l1' = -acc(|q - x|), where acc is the canonical blocked float32 sum of DESIGN.md section 4, so the scores are
+        bit-reproducible; a zero row under cosine scores NaN.  exclude_self: an id query leaves its own row out (rows
+        with identical values stay); vector queries exclude nothing.  Returns (ids int64 [Q, k], scores float32 [Q, k])
+        on the model's device, ordered as predict_topk's: score descending, then row id ascending, NaN last, -0.0 ==
+        +0.0; slots beyond the rows left hold id -1 and score -inf.  An id outside the table raises IndexError.  With an
+        initialised process group every rank selects over its row slice and the lists are merged (a collective: call it
+        on every rank with the same items)."""
+        if table not in ('entity', 'relation'):
+            raise ValueError("table must be 'entity' or 'relation', got %r" % (table,))
+        if metric not in _lib.SIM_IDS:
+            raise ValueError('metric must be one of %s, got %r' % (', '.join(_lib.SIM_IDS), metric))
+        if isinstance(k, bool) or int(k) != k or not 1 <= int(k) <= self.TOPK_MAX:
+            raise ValueError('k must be an integer in [1, %d], got %r' % (self.TOPK_MAX, k))
+        k = int(k)
+        X = self.entity_embedding if table == 'entity' else self.relation_embedding
+        rows, width = X.shape
+        arr = items.detach() if isinstance(items, torch.Tensor) else np.ascontiguousarray(items)
+        if arr.ndim == 1:
+            if arr.shape[0] and not _is_integer(arr):
+                raise ValueError('1-D items must be integer row ids, got dtype %s' % (arr.dtype,))
+        elif arr.ndim == 2:
+            if not (arr.dtype.is_floating_point if isinstance(arr, torch.Tensor)
+                    else np.issubdtype(arr.dtype, np.floating)):
+                raise ValueError('2-D items must be float query vectors [Q, %d], got dtype %s' % (width, arr.dtype))
+            if arr.shape[1] != width:
+                raise ValueError('query vectors of width %d, the %s table has width %d' % (arr.shape[1], table, width))
+        else:
+            raise ValueError('items must be 1-D row ids or 2-D query vectors, got %d dimensions' % arr.ndim)
+        dev = self._device()
+        st = _stream(dev)
+        by_id = arr.ndim == 1
+        if by_id:
+            src = torch.as_tensor(arr) if arr.shape[0] else torch.empty(0, dtype=torch.int64)
+            queries = src.to(device=dev, dtype=torch.int64).contiguous()
+        else:
+            queries = torch.as_tensor(arr).to(device=dev, dtype=torch.float32).contiguous()
+        nq = queries.shape[0]
+        ids = torch.empty((nq, k), dtype=torch.int64, device=dev)
+        scores = torch.empty((nq, k), dtype=torch.float32, device=dev)
+        if nq == 0:
+            return ids, scores
+        rank, world = _dist()
+        row_begin, row_end = shard_bounds(rows, rank, world, align=128)
+        desc = self._descriptor()
+        err = self._err_flag()
+        lib = _lib.load()
+        tab = _lib.TABLE_ENTITY if table == 'entity' else _lib.TABLE_RELATION
+        sim = _lib.SIM_IDS[metric]
+        xnorm = None
+        if metric == 'cosine':             # recomputed every call: training changes the tables, and it is one read
+            xnorm = self._buffer('nn_xnorm', rows, torch.float32, dev)
+            _lib.call("kge_similarity_norms", ctypes.byref(desc), tab, None, rows, _ptr(xnorm), st)
+        # the keys of this rank's slice, merged over the ranks below (one device: merged and decoded per chunk)
+        local = torch.empty((nq, k), dtype=torch.int64, device=dev) if world > 1 else None
+        chunk = 4096
+        for lo in range(0, nq, chunk):
+            q = queries[lo:lo + chunk]
+            Q = q.shape[0]
+            self_ids = None
+            if by_id:
+                qvec = self._buffer('nn_qvec', Q * width, torch.float32, dev)
+                _lib.call("kge_similarity_rows", ctypes.byref(desc), tab, _ptr(q), Q, _ptr(qvec), _ptr(err), st)
+                self_ids = q if exclude_self else None
+            else:
+                qvec = q
+            qnorm = None
+            if metric == 'cosine':
+                qnorm = self._buffer('nn_qnorm', Q, torch.float32, dev)
+                _lib.call("kge_similarity_norms", ctypes.byref(desc), tab, _ptr(qvec), Q, _ptr(qnorm), st)
+            sbytes = int(lib.kge_similarity_topk_scratch_bytes(ctypes.byref(desc), tab, Q, row_begin, row_end, k))
+            _lib.check(min(sbytes, 0))
+            scratch = self._buffer('nn_scratch', sbytes, torch.uint8, dev)
+            keys = local[lo:lo + Q] if local is not None else self._buffer('nn_keys', Q * k, torch.int64, dev)
+            events = self._ws.get('nn_events')               # tools/similarity_rate.py: CUDA events around select + merge
+            if events is not None:
+                ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                ev0.record()
+            _lib.call("kge_similarity_topk", ctypes.byref(desc), tab, sim, _ptr(qvec), _ptr(qnorm), _ptr(xnorm),
+                      _ptr(self_ids), Q, row_begin, row_end, k, _ptr(keys), _ptr(scratch), sbytes, st)
+            if local is None:
+                _lib.call("kge_eval_topk_merge", _ptr(keys), Q, 1, k, None, _ptr(ids[lo:lo + Q]),
+                          _ptr(scores[lo:lo + Q]), st)
+            if events is not None:
+                ev1.record()
+                events.append((ev0, ev1))
+        if local is not None:
+            import torch.distributed as dist
+            gloo = dist.get_backend() == 'gloo'          # gloo gathers host tensors only
+            mine = local.cpu() if gloo else local
+            parts = [torch.empty_like(mine) for _ in range(world)]
+            dist.all_gather(parts, mine)
+            lists = torch.stack(parts, dim=1).to(dev).contiguous()          # [Q, world, k]
+            _lib.call("kge_eval_topk_merge", _ptr(lists), nq, world, k, None, _ptr(ids), _ptr(scores), st)
+        self._raise_if_bad_index()                        # the call's one host sync
+        return ids, scores
+
     @staticmethod
     def test_step(model, test_triples, all_true_triples, args):
         '''
