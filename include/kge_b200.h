@@ -324,6 +324,32 @@ int kge_eval_filter_bits_lookup_dense(const int32_t *index_offsets, const int32_
                                       const int64_t *queries, int64_t Q, int mode, int64_t nentity, int64_t nrelation,
                                       uint32_t *filter_bits, void *stream);
 
+/* ---- path queries (a, r1/.../rL, ?) and (?, r1/.../rL, a): multi-hop questions ranked by the one-hop kernels ----
+ * anchors [Q] int64 entity ids; paths [Q, L] int64 hop ids: r in [0, nrelation) follows relation r, r + nrelation follows
+ * it inverted, -1 pads a row after its last hop (every row has at least one hop).
+ * kge_eval_path_query_vectors: qvec [Q, entity_dim], the path folded into one query vector with the non-contracted
+ *   primitives of kge_eval_query_vectors (tail-batch: row(a) through hops 1..L; head-batch: from row(a), -row(a) for
+ *   TransE and pRotatE, through hops L..1), so that a one-hop forward path gives that call's vector bit for bit.  It feeds
+ *   kge_eval_positive_scores, the count / stats entries and kge_eval_topk as a query vector of `mode`.  A bad anchor, hop
+ *   id or padding sets *err_flag (may be NULL) and folds a zero row.
+ * kge_eval_path_bits_dense / kge_eval_path_bits: bits [Q, ceil(nentity/32)] = the entities reachable from the anchor along
+ *   the path in the indexed triples (tail-batch: forward along hops 1..L; head-batch: backward from hop L), in the
+ *   filter_bits layout, by one traversal launch per hop over the bitmaps bits and pong (same size, distinct).  The tail
+ *   index ((h, r) -> tails, TAIL_BATCH build of kge_eval_filter_index_build or kge_eval_filter_bits_lookup's table) serves
+ *   forward tail-batch hops and inverse head-batch hops, the head index ((r, t) -> heads) the other two; an index may be
+ *   NULL (nkeys 0) when no hop of the call reads it.  answer_counts [Q] int32 (may be NULL): the size of each set.     */
+int kge_eval_path_query_vectors(const kge_model_t *m, int mode, const int64_t *anchors, const int64_t *paths, int64_t Q,
+                                int64_t L, float *qvec, int32_t *err_flag, void *stream);
+int kge_eval_path_bits_dense(const int32_t *tail_offsets, const int32_t *tail_entities, const int32_t *head_offsets,
+                             const int32_t *head_entities, const int64_t *anchors, const int64_t *paths, int64_t Q,
+                             int64_t L, int mode, int64_t nentity, int64_t nrelation, uint32_t *bits, uint32_t *pong,
+                             int32_t *answer_counts, void *stream);
+int kge_eval_path_bits(const int64_t *tail_keys, const int64_t *tail_offsets, const int32_t *tail_entities,
+                       int64_t tail_nkeys, const int64_t *head_keys, const int64_t *head_offsets,
+                       const int32_t *head_entities, int64_t head_nkeys, const int64_t *anchors, const int64_t *paths,
+                       int64_t Q, int64_t L, int mode, int64_t nentity, int64_t nrelation, uint32_t *bits, uint32_t *pong,
+                       int32_t *answer_counts, void *stream);
+
 /* ---- top-k link prediction: the k most plausible entities of every query (h, r, ?) / (?, r, t) ----
  * Scores are the canonical exact ones of kge_eval_count_ranks (bit-identical to that kernel and to the C oracle) for
  * every model; the [Q, nentity] score matrix is never formed.  Order: score descending, then entity id ascending; NaN

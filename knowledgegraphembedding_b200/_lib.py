@@ -109,6 +109,13 @@ PROTOTYPES = {
     "kge_eval_candidate_rank_stats": (c_int, [_M, c_int, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p,
                                               c_int64, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_void_p,
                                               c_void_p]),
+    "kge_eval_path_query_vectors": (c_int, [_M, c_int, c_void_p, c_void_p, c_int64, c_int64, c_void_p, c_void_p,
+                                            c_void_p]),
+    "kge_eval_path_bits_dense": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int64,
+                                         c_int, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "kge_eval_path_bits": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_int64,
+                                   c_void_p, c_void_p, c_int64, c_int64, c_int, c_int64, c_int64, c_void_p, c_void_p,
+                                   c_void_p, c_void_p]),
     "kge_eval_topk_scratch_bytes": (c_int64, [_M, c_int64, c_int64, c_int64, c_int]),
     "kge_eval_topk": (c_int, [_M, c_int, c_void_p, c_int64, c_void_p, c_void_p, c_int64, c_int64, c_int, c_void_p,
                               c_void_p, c_int64, c_void_p]),

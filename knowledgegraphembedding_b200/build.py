@@ -7,7 +7,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(CSRC, "libkge_b200.so")
 SOURCES = ["kge_train.cu", "kge_optim.cu", "kge_eval.cu", "kge_eval_gemm.cu", "kge_eval_topk.cu", "kge_eval_relation.cu",
-           "kge_eval_candidates.cu", "kge_sampler.cu", "kge_peer.cu", "kge_train_inst.cu"]
+           "kge_eval_candidates.cu", "kge_eval_path.cu", "kge_sampler.cu", "kge_peer.cu", "kge_train_inst.cu"]
 HEADERS = ["kge_common.cuh", "kge_rows.cuh", "kge_adam.cuh", "kge_eval_tile.cuh", "kge_train_args.cuh",
            "kge_train_kernels.cuh",
            "kge_train_split.cuh", "kge_train_launch.cuh", "kge_math.h", os.path.join("..", "..", "include", "kge_b200.h")]

@@ -956,15 +956,19 @@ class KGEModel(nn.Module):
         return self._entity_rank_counts(test_triples, all_true_triples, mode, query_chunk, exact, True)[0]
 
     def _entity_rank_counts(self, test_triples, all_true_triples, mode, query_chunk, exact, stats,
-                            return_scores=False, return_approx=False):
+                            return_scores=False, return_approx=False, path=None):
         """The query loop of filtered_ranks (stats=False: int64 counts [len]) and rank_statistics (stats=True: int64
-        [len, 6]), with the [len, nentity] score dumps of filtered_ranks (None when not asked for)."""
+        [len, 6]), with the [len, nentity] score dumps of filtered_ranks (None when not asked for).  path (a _PathQueries
+        of path_rank_statistics): its answer sets and folded vectors replace the filter bitmap and the query vectors of
+        each chunk; test_triples then only carries the positives, and the answer counts are left in path.answer_counts."""
         dev = self._device()
         st = _stream(dev)
         nentity, nrelation = self.entity_embedding.shape[0], self.relation_embedding.shape[0]
-        index = self._filter_index(all_true_triples, nentity, nrelation)
         cached = self._ws.get('queries_np')                  # test_step ranks the same list in both modes
-        if cached is not None and cached[0] is test_triples and cached[1] == len(test_triples) and cached[3].device == dev:
+        if path is not None:
+            queries_all = np.asarray(test_triples, dtype=np.int64).reshape(-1, 3)
+            queries_dev = torch.from_numpy(queries_all).to(dev, non_blocking=True)
+        elif cached is not None and cached[0] is test_triples and cached[1] == len(test_triples) and cached[3].device == dev:
             queries_all, queries_dev = cached[2], cached[3]
         else:
             queries_all = np.asarray(test_triples, dtype=np.int64).reshape(-1, 3)
@@ -972,7 +976,8 @@ class KGEModel(nn.Module):
             self._ws['queries_np'] = (test_triples, len(test_triples), queries_all, queries_dev)
         if mode not in ('head-batch', 'tail-batch'):
             raise ValueError('negative batch mode %s not supported' % mode)       # dataloader.py:147
-        ftab = self._filter_tables(index, mode, dev, st)
+        if path is None:
+            ftab = self._filter_tables(self._filter_index(all_true_triples, nentity, nrelation), mode, dev, st)
         rank, world = _dist()
         ent_begin, ent_end = shard_bounds(nentity, rank, world, align=128)
         desc = self._descriptor()
@@ -989,12 +994,13 @@ class KGEModel(nn.Module):
         two_stage = not exact and ((self.model_name == 'RotatE' and self.entity_dim % 8 == 0) or
                                    (self.model_name == 'pRotatE' and self.entity_dim % 4 == 0))
         nchunks = (queries_all.shape[0] + query_chunk - 1) // query_chunk
-        # one int32 buffer [rank counts | per-chunk (ambiguous pairs, overflow flag)]: a single all-reduce and a single
-        # read-back per call
+        # one int32 buffer [rank counts | per-chunk (ambiguous pairs, overflow flag) | path answer counts]: a single
+        # all-reduce and a single read-back per call
         nq_all = queries_all.shape[0]
         ncol = self.RANK_STATS if stats else 1
-        tally = torch.zeros(nq_all * ncol + 2 * max(nchunks, 1), dtype=torch.int32, device=dev)
-        amb_counts = tally[nq_all * ncol:].view(-1, 2) if (gemm or two_stage) else None
+        namb = 2 * max(nchunks, 1)
+        tally = torch.zeros(nq_all * ncol + namb + (nq_all if path is not None else 0), dtype=torch.int32, device=dev)
+        amb_counts = tally[nq_all * ncol:nq_all * ncol + namb].view(-1, 2) if (gemm or two_stage) else None
         if gemm:
             nE = self.entity_embedding.numel()
             ehi = self._buffer('gemm_ehi', nE, torch.float32, dev)
@@ -1016,14 +1022,18 @@ class KGEModel(nn.Module):
             qvec = self._buffer('qvec', Q * self.entity_dim, torch.float32, dev)
             pos = self._buffer('pos_score', Q, torch.float32, dev)
             counts = counts_all[lo * ncol:(lo + Q) * ncol]
+            if path is not None:                            # answer sets + folded paths (rank 0 counts the answers)
+                answers = tally[nq_all * ncol + namb + lo:] if rank == 0 else None
+                self._path_chunk(path, lo, Q, m, desc, bits, qvec, answers, err, st)
             # filter bitmap of the chunk, looked up on the device in the resident index (dataloader.py:134-154)
-            if ftab[0] == 'dense':
+            elif ftab[0] == 'dense':
                 _lib.call("kge_eval_filter_bits_lookup_dense", _ptr(ftab[1]), _ptr(ftab[2]), _ptr(queries), Q, m, nentity,
                           nrelation, _ptr(bits), st)
             else:
                 _lib.call("kge_eval_filter_bits_lookup", _ptr(ftab[1]), _ptr(ftab[2]), _ptr(ftab[3]), ftab[4],
                           _ptr(queries), Q, m, nentity, nrelation, _ptr(bits), st)
-            _lib.call("kge_eval_query_vectors", ctypes.byref(desc), m, _ptr(queries), Q, _ptr(qvec), _ptr(err), st)
+            if path is None:
+                _lib.call("kge_eval_query_vectors", ctypes.byref(desc), m, _ptr(queries), Q, _ptr(qvec), _ptr(err), st)
             _lib.call("kge_eval_positive_scores", ctypes.byref(desc), m, _ptr(qvec), _ptr(queries), Q, _ptr(phase),
                       _ptr(pos), st)
             events = self._ws.get('eval_events')            # bench.py: CUDA events around the dominant kernel
@@ -1073,11 +1083,18 @@ class KGEModel(nn.Module):
         counts = host[:nq_all * ncol].astype(np.int64)
         if stats:
             counts = counts.reshape(nq_all, ncol)
+        if path is not None:
+            path.answer_counts = host[nq_all * ncol + namb:].astype(np.int64)
         if amb_counts is not None:
-            amb_host = host[nq_all * ncol:].reshape(-1, 2)
+            amb_host = host[nq_all * ncol:nq_all * ncol + namb].reshape(-1, 2)
             self._ws['gemm_last_ambiguous' if gemm else 'two_stage_last_ambiguous'] = int(amb_host[:, 0].sum())
             for ci in np.nonzero(amb_host[:, 1])[0]:         # ambiguous list overflowed: exact kernel for that chunk
                 lo = int(ci) * query_chunk
+                if path is not None:
+                    counts[lo:lo + query_chunk] = self._entity_rank_counts(
+                        queries_all[lo:lo + query_chunk], None, mode, query_chunk, True, stats,
+                        path=path.slice(lo, lo + query_chunk))[0]
+                    continue
                 chunk = [tuple(int(v) for v in row) for row in queries_all[lo:lo + query_chunk]]
                 counts[lo:lo + query_chunk] = self._entity_rank_counts(chunk, all_true_triples, mode, query_chunk, True,
                                                                        stats)[0]
@@ -1223,6 +1240,13 @@ class KGEModel(nn.Module):
             arr = np.array(queries, dtype=np.int64).reshape(-1, 3)
             arr[:, 0 if head else 2] = 0         # unused; an out-of-range value would set the bad-index flag
             queries_dev = torch.from_numpy(arr).to(dev, non_blocking=True)
+        return self._topk_chunks(queries_dev, mode, k, exclude_triples)
+
+    def _topk_chunks(self, queries_dev, mode, k, exclude_triples, path=None, chunk=4096):
+        """The chunk loop of predict_topk; path (a _PathQueries of predict_path_topk): its folded vectors and, with
+        exclude_triples, its answer sets replace the query vectors and the exclusion bitmap of each chunk."""
+        dev = self._device()
+        st = _stream(dev)
         nq = queries_dev.shape[0]
         ids = torch.empty((nq, k), dtype=torch.int64, device=dev)
         scores = torch.empty((nq, k), dtype=torch.float32, device=dev)
@@ -1230,7 +1254,7 @@ class KGEModel(nn.Module):
             return ids, scores
         nentity, nrelation = self.entity_embedding.shape[0], self.relation_embedding.shape[0]
         ftab = None
-        if exclude_triples is not None:
+        if exclude_triples is not None and path is None:
             ftab = self._filter_tables(self._filter_index(exclude_triples, nentity, nrelation), mode, dev, st)
         rank, world = _dist()
         ent_begin, ent_end = shard_bounds(nentity, rank, world, align=128)
@@ -1245,12 +1269,15 @@ class KGEModel(nn.Module):
         m = _lib.MODE_IDS[mode]
         # the keys of this rank's slice, merged over the ranks below (one device: merged and decoded per chunk)
         local = torch.empty((nq, k), dtype=torch.int64, device=dev) if world > 1 else None
-        chunk = 4096
         for lo in range(0, nq, chunk):
             q = queries_dev[lo:lo + chunk]
             Q = q.shape[0]
             bits = None
-            if ftab is not None:
+            if path is not None:
+                bits = self._buffer('topk_bits', Q * words, torch.int32, dev) if exclude_triples is not None else None
+                qvec = self._buffer('topk_qvec', Q * self.entity_dim, torch.float32, dev)
+                self._path_chunk(path, lo, Q, m, desc, bits, qvec, None, err, st)
+            elif ftab is not None:
                 bits = self._buffer('topk_bits', Q * words, torch.int32, dev)
                 if ftab[0] == 'dense':
                     _lib.call("kge_eval_filter_bits_lookup_dense", _ptr(ftab[1]), _ptr(ftab[2]), _ptr(q), Q, m, nentity,
@@ -1258,8 +1285,9 @@ class KGEModel(nn.Module):
                 else:
                     _lib.call("kge_eval_filter_bits_lookup", _ptr(ftab[1]), _ptr(ftab[2]), _ptr(ftab[3]), ftab[4],
                               _ptr(q), Q, m, nentity, nrelation, _ptr(bits), st)
-            qvec = self._buffer('topk_qvec', Q * self.entity_dim, torch.float32, dev)
-            _lib.call("kge_eval_query_vectors", ctypes.byref(desc), m, _ptr(q), Q, _ptr(qvec), _ptr(err), st)
+            if path is None:
+                qvec = self._buffer('topk_qvec', Q * self.entity_dim, torch.float32, dev)
+                _lib.call("kge_eval_query_vectors", ctypes.byref(desc), m, _ptr(q), Q, _ptr(qvec), _ptr(err), st)
             sbytes = int(lib.kge_eval_topk_scratch_bytes(ctypes.byref(desc), Q, ent_begin, ent_end, k))
             _lib.check(min(sbytes, 0))
             scratch = self._buffer('topk_scratch', sbytes, torch.uint8, dev)
@@ -1286,6 +1314,103 @@ class KGEModel(nn.Module):
             _lib.call("kge_eval_topk_merge", _ptr(lists), nq, world, k, None, _ptr(ids), _ptr(scores), st)
         self._raise_if_bad_index()                        # the call's one host sync
         return ids, scores
+
+    # ------------------------------------------------------------------------------------------ path queries
+    def path_rank_statistics(self, anchors, paths, answers, all_true_triples, mode, query_chunk=4096, exact=False,
+                             return_answer_counts=False):
+        """Rank statistics of path queries (Guu et al. 2015; the 1p/2p/3p projection chains of complex-query benchmarks):
+        int64 numpy [Q, 6] with the columns, tie rule and NaN / -0.0 handling of rank_statistics, where a candidate is
+        filtered when it is in the query's answer set.
+
+        anchors: int [Q] entity ids.  paths: int [Q, L] hop ids: r in [0, nrelation) follows relation r, r + nrelation
+        follows it inverted, -1 pads a row after its last hop (every row has at least one hop).  answers: int [Q], the
+        entity ranked.  mode 'tail-batch' asks (a, r1/.../rL, ?), the entities reached from a along the path; 'head-batch'
+        asks (?, r1/.../rL, a), the entities x with x -r1-> ... -rL-> a.  The path is folded into one query vector
+        (DESIGN.md section 3.13; one hop forward gives rank_statistics' numbers bit for bit) and the answer set is the
+        breadth-first traversal of the path in all_true_triples, on the device.  The counting path is rank_statistics'
+        (exact=True: the exact tile kernel).  return_answer_counts: also int64 [Q], the size of every answer set (the mean
+        quantile of Guu et al. needs it).  A bad anchor, hop id, padding or answer raises IndexError.  With an initialised
+        process group every rank counts over its entity slice and the tallies are all-reduced (a collective: call it on
+        every rank)."""
+        if isinstance(query_chunk, bool) or int(query_chunk) != query_chunk or int(query_chunk) < 1:
+            raise ValueError('query_chunk must be a positive integer, got %r' % (query_chunk,))
+        path, queries = self._path_queries(anchors, paths, mode, all_true_triples, answers)
+        # two [chunk, nentity / 32] bitmaps (ping-pong of the traversal) stay within _CAND_BITS_BUDGET
+        chunk = max(1, min(int(query_chunk), self._CAND_BITS_BUDGET // (8 * ((self.nentity + 31) // 32))))
+        stats = self._entity_rank_counts(queries, None, mode, chunk, exact, True, path=path)[0]
+        return (stats, path.answer_counts) if return_answer_counts else stats
+
+    def predict_path_topk(self, anchors, paths, mode, k=10, exclude_triples=None):
+        """The k most plausible answers of every path query, best first: (ids int64 [Q, k], scores float32 [Q, k]) on the
+        model's device, with the order, scores and empty slots of predict_topk.  anchors, paths and mode as in
+        path_rank_statistics; exclude_triples: optional list of true triples whose answer set along each path is left
+        out.  A bad anchor, hop id or padding raises IndexError.  With an initialised process group every rank selects
+        over its entity slice and the lists are merged (a collective: call it on every rank)."""
+        if isinstance(k, bool) or int(k) != k or not 1 <= int(k) <= self.TOPK_MAX:
+            raise ValueError('k must be an integer in [1, %d], got %r' % (self.TOPK_MAX, k))
+        path, _ = self._path_queries(anchors, paths, mode, exclude_triples)
+        chunk = 4096
+        if exclude_triples is not None:
+            chunk = max(1, min(chunk, self._CAND_BITS_BUDGET // (8 * ((self.nentity + 31) // 32))))
+        return self._topk_chunks(path.anchors, mode, int(k), exclude_triples, path=path, chunk=chunk)
+
+    def _path_queries(self, anchors, paths, mode, triples, answers=None):
+        """(_PathQueries on the device, queries [Q, 3] int64 numpy with the answers in the mode's positive column or None)
+        from the user's arrays; the filter indexes of `triples` the traversal reads are made resident."""
+        if mode not in ('head-batch', 'tail-batch'):
+            raise ValueError('negative batch mode %s not supported' % mode)
+        host = [np.asarray(x.detach().cpu() if isinstance(x, torch.Tensor) else x) for x in (anchors, paths)]
+        a, p = host
+        if a.ndim != 1 or p.ndim != 2 or p.shape[0] != a.shape[0] or p.shape[1] < 1 or \
+                (a.size and not _is_integer(a)) or (p.size and not _is_integer(p)):
+            raise ValueError('anchors must be integer ids [Q] and paths integer hop ids [Q, L >= 1], got %s %s and %s %s'
+                             % (a.dtype, tuple(a.shape), p.dtype, tuple(p.shape)))
+        a, p = a.astype(np.int64), np.ascontiguousarray(p, dtype=np.int64)
+        nentity, nrelation = self.entity_embedding.shape[0], self.relation_embedding.shape[0]
+        queries = None
+        if answers is not None:
+            t = np.asarray(answers.detach().cpu() if isinstance(answers, torch.Tensor) else answers)
+            if t.shape != a.shape or (t.size and not _is_integer(t)):
+                raise ValueError('answers must be integer ids [%d], got %s %s' % (a.shape[0], t.dtype, tuple(t.shape)))
+            if t.size and (t.min() < 0 or t.max() >= nentity):
+                raise IndexError('answer id outside the entity table')
+            queries = np.zeros((a.shape[0], 3), dtype=np.int64)
+            queries[:, 0 if mode == 'head-batch' else 2] = t
+        dev = self._device()
+        st = _stream(dev)
+        tables = None
+        if triples is not None:
+            held = self._filter_index(triples, nentity, nrelation)
+            forward, inverse = bool(((p >= 0) & (p < nrelation)).any()), bool((p >= nrelation).any())
+            if mode == 'head-batch':
+                forward, inverse = inverse, forward          # as index readers: head-batch walks the path backwards
+            tables = (self._filter_tables(held, 'tail-batch', dev, st) if forward else None,
+                      self._filter_tables(held, 'head-batch', dev, st) if inverse else None)
+        return _PathQueries(torch.from_numpy(a).to(dev), torch.from_numpy(p).to(dev), tables), queries
+
+    def _path_chunk(self, path, lo, Q, m, desc, bits, qvec, answer_counts, err, st):
+        """Queries [lo, lo + Q) of `path`: their folded vectors into qvec and, when bits is given, their answer sets into
+        bits (answer_counts: int32 [Q] set sizes, or None)."""
+        anchors, paths = path.anchors[lo:lo + Q], path.paths[lo:lo + Q]
+        L = paths.shape[1]
+        _lib.call("kge_eval_path_query_vectors", ctypes.byref(desc), m, _ptr(anchors), _ptr(paths), Q, L, _ptr(qvec),
+                  _ptr(err), st)
+        if bits is None:
+            return
+        nentity, nrelation = self.entity_embedding.shape[0], self.relation_embedding.shape[0]
+        pong = self._buffer('path_pong', Q * ((nentity + 31) // 32), torch.int32, bits.device)
+        tail, head = path.tables
+        layouts = {t[0] for t in (tail, head) if t is not None}
+        if layouts == {'sorted'}:
+            name = "kge_eval_path_bits"
+            index = [v for t in (tail, head) for v in ((_ptr(t[1]), _ptr(t[2]), _ptr(t[3]), t[4]) if t else (None,) * 3 + (0,))]
+        elif layouts <= {'dense'}:
+            name = "kge_eval_path_bits_dense"
+            index = [_ptr(t[i]) if t else None for t in (tail, head) for i in (1, 2)]
+        else:        # KGE_FILTER_HOST_INDEX changed between two calls on the same list
+            raise ValueError('the two filter indexes of this triple list have different layouts; pass a new list object')
+        _lib.call(name, *index, _ptr(anchors), _ptr(paths), Q, L, m, nentity, nrelation, _ptr(bits), _ptr(pong),
+                  _ptr(answer_counts), st)
 
     # ------------------------------------------------------------------------------------------ relation prediction
     def _relation_filter_table(self, held, dev):
@@ -1626,6 +1751,18 @@ def metrics_from_ranks(ranks):
         'HITS@10': (ranking <= 10).astype(np.float64),
     }
     return {name: sum(values.tolist()) / len(ranking) for name, values in per_query.items()}
+
+
+class _PathQueries:
+    """Path queries on the device (anchors int64 [Q], hop ids int64 [Q, L]) and the resident filter indexes their answer
+    sets are traversed in, (tail index, head index) with None for one no hop reads, or None without answer sets."""
+
+    def __init__(self, anchors, paths, tables):
+        self.anchors, self.paths, self.tables = anchors, paths, tables
+        self.answer_counts = None            # int64 numpy [Q], left here by KGEModel._entity_rank_counts
+
+    def slice(self, lo, hi):
+        return _PathQueries(self.anchors[lo:hi], self.paths[lo:hi], self.tables)
 
 
 class _NamedView:
