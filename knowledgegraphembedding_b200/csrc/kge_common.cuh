@@ -183,12 +183,24 @@ __device__ __forceinline__ float sigmoid(float x) {
   float e = expf(-fabsf(x));
   return x >= 0.f ? 1.f / (1.f + e) : e / (1.f + e);
 }
+// 2^x and 1/x on the MUFU pipe, one instruction each; flush-to-zero (without it, ex2 is wrapped in a subnormal range
+// check and two rescaling multiplies)
+__device__ __forceinline__ float ex2_ftz(float x) {
+  float r;
+  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
+  return r;
+}
+__device__ __forceinline__ float rcp_ftz(float x) {
+  float r;
+  asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
+  return r;
+}
+constexpr float kLog2e = 1.44269504088896341f;
 // sigmoid on the MUFU pipe (ex2 + rcp, ~2^-21 relative): the per-candidate softmax weight of the train kernel sits on the
 // warp's serial path, where the IEEE division of sigmoid() costs ~40 cycles of latency
 __device__ __forceinline__ float sigmoid_fast(float x) {
-  const float e = __expf(-fabsf(x));
-  float r;
-  asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(1.f + e));
+  const float e = ex2_ftz(-kLog2e * fabsf(x));
+  const float r = rcp_ftz(1.f + e);
   return x >= 0.f ? r : e * r;
 }
 #endif

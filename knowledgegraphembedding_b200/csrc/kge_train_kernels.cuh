@@ -250,7 +250,7 @@ __device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {
 __device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
 }
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
+__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {   // bar: shared-window address
   asm volatile(
       "{\n"
       ".reg .pred p;\n"
@@ -259,10 +259,11 @@ __device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
       "@p bra DONE_%=;\n"
       "bra WAIT_%=;\n"
       "DONE_%=:\n"
-      "}\n" ::"r"(smem_u32(bar)),
+      "}\n" ::"r"(bar),
       "r"(parity)
       : "memory");
 }
+__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) { mbar_wait(smem_u32(bar), parity); }
 __device__ __forceinline__ void bulk_g2s(void *dst, const void *src, uint32_t bytes, uint64_t *bar) {
   asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
                    smem_u32(dst)),
@@ -277,6 +278,37 @@ __device__ __forceinline__ void bulk_g2s_hint(void *dst, const void *src, uint32
       "l"(src), "r"(bytes), "r"(smem_u32(bar)), "l"(pol)
       : "memory");
 }
+
+// expect_tx of 2 x `bytes` (NCOPY 2) or `bytes` (NCOPY 1) on `bar`, and the copies src0 -> dst0 [, src1 -> dst1],
+// issued by one lane that elect.sync picks from the whole (converged) warp.  Every lane passes the same operands (a
+// shuffled id): under elect.sync ptxas moves them to uniform registers once, where a `lane == 0` branch made it wrap
+// every copy in a re-election loop (ELECT / R2UR / BRA.U.ANY) for operands it could not prove uniform.
+// HINT: the copies carry the L2 cache policy `pol`.
+#define KGE_BULK_ELECT_HEAD "{\n.reg .pred p;\nelect.sync _|p, 0xffffffff;\n@p mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;\n"
+#define KGE_BULK_ELECT_COPY(D, S) \
+  "@p cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [" D "], [" S "], %4, [%0];\n"
+#define KGE_BULK_ELECT_COPY_HINT(D, S) \
+  "@p cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [" D "], [" S "], %4, [%0], %7;\n"
+template <int NCOPY, bool HINT>
+__device__ __forceinline__ void bulk_g2s_warp(uint32_t bar, uint32_t dst0, const void *src0, uint32_t dst1,
+                                              const void *src1, uint32_t bytes, uint64_t pol = 0) {
+  static_assert(NCOPY == 1 || NCOPY == 2, "one or two copies");
+  if constexpr (HINT && NCOPY == 2)
+    asm volatile(KGE_BULK_ELECT_HEAD KGE_BULK_ELECT_COPY_HINT("%2", "%3") KGE_BULK_ELECT_COPY_HINT("%5", "%6") "}\n"
+                 ::"r"(bar), "r"(bytes * NCOPY), "r"(dst0), "l"(src0), "r"(bytes), "r"(dst1), "l"(src1), "l"(pol) : "memory");
+  else if constexpr (HINT)
+    asm volatile(KGE_BULK_ELECT_HEAD KGE_BULK_ELECT_COPY_HINT("%2", "%3") "}\n"
+                 ::"r"(bar), "r"(bytes * NCOPY), "r"(dst0), "l"(src0), "r"(bytes), "r"(dst1), "l"(src1), "l"(pol) : "memory");
+  else if constexpr (NCOPY == 2)
+    asm volatile(KGE_BULK_ELECT_HEAD KGE_BULK_ELECT_COPY("%2", "%3") KGE_BULK_ELECT_COPY("%5", "%6") "}\n"
+                 ::"r"(bar), "r"(bytes * NCOPY), "r"(dst0), "l"(src0), "r"(bytes), "r"(dst1), "l"(src1), "l"(pol) : "memory");
+  else
+    asm volatile(KGE_BULK_ELECT_HEAD KGE_BULK_ELECT_COPY("%2", "%3") "}\n"
+                 ::"r"(bar), "r"(bytes * NCOPY), "r"(dst0), "l"(src0), "r"(bytes), "r"(dst1), "l"(src1), "l"(pol) : "memory");
+}
+#undef KGE_BULK_ELECT_HEAD
+#undef KGE_BULK_ELECT_COPY
+#undef KGE_BULK_ELECT_COPY_HINT
 
 template <int MODEL, bool HEAD>
 __global__ void __launch_bounds__(512, 1) row_kernel_tma(const RowArgs a) {

@@ -124,6 +124,7 @@ __global__ void __launch_bounds__(split_warps(op_is_complex(op_of(MODEL, HEAD)),
   uint64_t *bars = sbars + 2;
   const uint32_t halfbytes = (uint32_t)a.d * 4u;
   uint64_t *gbars = bars + D * warp;                       // this group's mbarriers
+  const uint32_t gbars_s = smem_u32(gbars), slots_s = smem_u32(slots);   // (their shared-window addresses)
   uint32_t par = 0;                                         // phase parity of every slot's mbarrier (bit s)
   float *xch = reinterpret_cast<float *>(bars + D * nwarps) + 4 * warp;      // [2 parities][2 halves] partial scores
   int *parks = reinterpret_cast<int *>(reinterpret_cast<float *>(bars + D * nwarps) + 4 * nwarps);
@@ -155,8 +156,11 @@ __global__ void __launch_bounds__(split_warps(op_is_complex(op_of(MODEL, HEAD)),
   bool primed = false;                                     // the first D candidates of the current row are already issued
   // candidate ids of this warp, 32 at a time (see issue()): the current window, the next window of the same row
   // (fetched 24 candidates ahead) and the first window of the next row (fetched a whole row ahead) -- the id loads
-  // never sit in front of a bulk copy (ncu r2d: they did, ~1 us of long-scoreboard stall per 32 candidates and warp)
-  int64_t ids = 0, ids_nxt = 0, ids_next_row = 0;
+  // never sit in front of a bulk copy (ncu r2d: they did, ~1 us of long-scoreboard stall per 32 candidates and warp).
+  // The current window is held clamped as int32 row indices: the single-read path requires nentity < 2^31
+  // (split_path_shape_ok), and the row's source address is then one wide multiply-add of the shuffled index.
+  int idw = 0;
+  int64_t ids_nxt = 0, ids_next_row = 0;
   bool next_row_ready = false;
   int ids_base = -32;
   int cand_rl = 0;
@@ -202,8 +206,11 @@ __global__ void __launch_bounds__(split_warps(op_is_complex(op_of(MODEL, HEAD)),
 
     // candidate ids of this warp (n = warp + j * nwarps), fetched 32 at a time with one load per lane and handed out
     // by shuffle: no dependent global load sits in front of a bulk copy
+    // Called by the whole warp (converged).  Per candidate: one shuffle of the window's index and the elected copy issue;
+    // the per-id work runs once per window, one candidate per lane.
     auto issue = [&](int s, int j) {                       // j-th candidate of this warp (of the row `cand` points to)
       if (j >= ids_base + 32) {                            // (j is a multiple of 32 here)
+        int64_t ids;
         if (j == 0) {
           if (next_row_ready) {
             ids = ids_next_row;
@@ -215,28 +222,29 @@ __global__ void __launch_bounds__(split_warps(op_is_complex(op_of(MODEL, HEAD)),
           ids = ids_nxt;
         }
         ids_base = j;
-        // the window becomes current: clamp its ids once (like every gather) and keep an int32 copy on the device --
+        // the window becomes current: every lane clamps its id once (like every gather), adds it to the histogram of
+        // the entity-major pass (one warp-wide reduction for 32 candidates) and keeps an int32 copy on the device --
         // the counting sort reads that instead of the caller's int64 array, which may live in pinned HOST memory
         // (zero-copy batches: this kernel's prefetched window loads are then the only PCIe reads of the ids)
         const int nw = warp + (j + lane) * nwarps;
         if (nw < a.N) {
           if ((uint64_t)ids >= (uint64_t)a.nentity) { if (a.err) *a.err = 1; ids = 0; }
-          if (ws.ids32 && hw == 0) ws.ids32[(size_t)cand_rl * a.N + nw] = (int)ids;
+          if (hw == 0) {
+            atomicAdd(ws.cnt + ids, 1);
+            if (ws.ids32) ws.ids32[(size_t)cand_rl * a.N + nw] = (int)ids;
+          }
         }
+        idw = (int)ids;
       }
       if (j == ids_base + 8) {                             // next window of this row, 24 candidates ahead of its use
         const int n = warp + (ids_base + 32 + lane) * nwarps;
         ids_nxt = n < a.N ? cand[n] : 0;
       }
-      const int64_t id = __shfl_sync(0xffffffffu, ids, j - ids_base);
-      if (lane == 0 && hw == 0) {
-        atomicAdd(ws.cnt + id, 1);                        // histogram for the entity-major pass
-        uint64_t *bar = gbars + s;
-        float *dst = slots + (size_t)s * HS;
-        const float *src = a.E + id * a.De;
-        mbar_expect_tx(bar, halfbytes * H);
-        bulk_g2s_hint(dst, src, halfbytes, bar, pol_e);
-        if constexpr (CPLX) bulk_g2s_hint(dst + DP, src + a.d, halfbytes, bar, pol_e);
+      const int id = __shfl_sync(0xffffffffu, idw, j - ids_base);
+      if (hw == 0) {
+        const float *src = a.E + (size_t)(uint32_t)id * (uint32_t)a.De;
+        const uint32_t dst = slots_s + (uint32_t)(s * HS) * 4u;
+        bulk_g2s_warp<H, true>(gbars_s + 8u * s, dst, src, dst + DP * 4u, src + a.d, halfbytes, pol_e);
       }
     };
     if (!primed) {
@@ -286,13 +294,14 @@ __global__ void __launch_bounds__(split_warps(op_is_complex(op_of(MODEL, HEAD)),
       }
     }
     {
+      const bool lead = lane == 0 && hw == 0, timed = a.phase_cycles && tid == 0;
       int it = 0;
       for (int n = warp; n < a.N; n += nwarps, ++it) {
         const int s = cons;
         cons = cons + 1 == D ? 0 : cons + 1;
-        { const long long tw_ = (a.phase_cycles && tid == 0) ? clock64() : 0;
-          mbar_wait(gbars + s, (par >> s) & 1u);
-          if (a.phase_cycles && tid == 0) atomicAdd(a.phase_cycles + 6, (unsigned long long)(clock64() - tw_)); }
+        { const long long tw_ = timed ? clock64() : 0;
+          mbar_wait(gbars_s + 8u * s, (par >> s) & 1u);
+          if (timed) atomicAdd(a.phase_cycles + 6, (unsigned long long)(clock64() - tw_)); }
         par ^= 1u << s;
         float *xl = slots + (size_t)s * HS + c0 * 128 + lane * V;
         // sweep 1: element values -> score; u = d(value)/dq stays in registers (VAR >= 1) or is parked in the slot
@@ -411,10 +420,7 @@ __global__ void __launch_bounds__(split_warps(op_is_complex(op_of(MODEL, HEAD)),
             if (n + D * nwarps < a.N) issue(s, it + D);
           }
           const float sv = finish_score<MODEL>(part, a.gamma, modulus);
-          if (lane == 0 && hw == 0) {
-            sc[n] = sv;
-            if (a.score_out) a.score_out[(int64_t)rl * a.N + n] = sv;
-          }
+          if (lead) sc[n] = sv;                            // (score_out is written from sc after the loop)
           if (adversarial) {                               // online softmax: weight relative to the running max
             const float z = sv * a.alpha;
             if (z > Mw) {
@@ -426,7 +432,8 @@ __global__ void __launch_bounds__(split_warps(op_is_complex(op_of(MODEL, HEAD)),
                 for (int h = 0; h < H; ++h) { acc[i][h][0] = mul2(acc[i][h][0], r2); acc[i][h][1] = mul2(acc[i][h][1], r2); }
               Mw = z;
             }
-            coef = __expf(z - Mw) * sigmoid_fast(sv);      // (2 ulp-level approximations: weights enter dL/dq at 1e-6)
+            // (2 ulp-level approximations: weights enter dL/dq at 1e-6; the two ex2 are independent MUFU instructions)
+            coef = ex2_ftz(kLog2e * (z - Mw)) * sigmoid_fast(sv);
           } else {
             coef = sigmoid_fast(sv);                       // uniform negatives: w = 1/N applied at the end
           }
@@ -503,6 +510,7 @@ __global__ void __launch_bounds__(split_warps(op_is_complex(op_of(MODEL, HEAD)),
       for (int n = tid; n < a.N; n += blockDim.x) {
         const float w = gg[n] / zsum;
         const float sv = sc[n];
+        if (a.score_out) a.score_out[(int64_t)rl * a.N + n] = sv;
         lacc += w * log_sigmoid(-sv);
         const float g = 0.5f * u * w * sigmoid(sv);
         store_all(a.mir, gout + n, g);
@@ -708,12 +716,11 @@ __global__ void __launch_bounds__(entity_warps(S, FUSED) * 32, 1) entity_kernel(
   constexpr int slot_floats = H * HSTR;
   // per warp a ring of D slots (D = a.depth, 2..4: the bytes in flight per SM are what hides the L2 latency of the q
   // rows -- ncu r2b: 45 % of the instructions of the depth-2 kernel were mbarrier polls); layout
-  // [slots: nwarps x D | mbarriers: nwarps x D | (dL/ds, perm entry) of the pair in each slot: nwarps x D]
+  // [slots: nwarps x D | mbarriers: nwarps x D] (the launcher sizes 16 bytes per slot for the mbarrier)
   const int D = a.depth;
   float *slots = smem + (size_t)(D * warp) * slot_floats;
   uint64_t *bars = reinterpret_cast<uint64_t *>(smem + (size_t)(D * nwarps) * slot_floats) + D * warp;
-  float2 *meta = reinterpret_cast<float2 *>(reinterpret_cast<uint64_t *>(smem + (size_t)(D * nwarps) * slot_floats) +
-                                            D * nwarps) + D * warp;      // FUSED: perm entry < 0 = direct gradient row
+  const uint32_t slots_s = smem_u32(slots), bars_s = smem_u32(bars);   // (their shared-window addresses)
   uint32_t par = 0;                                         // phase parity of every slot's mbarrier (bit s)
   const int nunits = a.d / V;
   const float modulus = MODEL == KGE_PROTATE ? __ldg(a.modulus) : 1.f;
@@ -748,28 +755,26 @@ __global__ void __launch_bounds__(entity_warps(S, FUSED) * 32, 1) entity_kernel(
     const uint32_t segbytes = (uint32_t)ucnt * V * 4u;
 
     // (row index, dL/ds) of the entity's pairs are fetched 32 at a time, one coalesced load per lane, and handed out
-    // by shuffle: no dependent global load sits in front of a bulk copy
-    int prow = 0;
-    float pg = 0.f;
+    // by shuffle: no dependent global load sits in front of a bulk copy.  Two windows stay live: (prow, pg) holds pairs
+    // pbase .. pbase + 31, which the copies are issued from, and (prow0, pg0) the 32 before, which the consumer -- D
+    // pairs behind the copies -- may still be reading.
+    int prow = 0, prow0 = 0;
+    float pg = 0.f, pg0 = 0.f;
     int pbase = beg - 32;                                   // first pair held in (prow, pg)
     auto refill = [&](int i) {
       pbase = i;
+      prow0 = prow; pg0 = pg;
       prow = i + lane < end ? a.perm[i + lane] : 0;
       pg = i + lane < end ? a.gsorted[i + lane] : 0.f;
     };
+    // called by the whole warp (converged): one shuffle, then the elected copy issue
     auto issue = [&](int s, int i) {
       if (i >= pbase + 32) refill(i);
       const int row = __shfl_sync(0xffffffffu, prow, i - pbase);
-      const float g = __shfl_sync(0xffffffffu, pg, i - pbase);
-      if (lane == 0) {
-        meta[s] = make_float2(g, __int_as_float(row));
-        uint64_t *bar = bars + s;
-        float *dst = slots + (size_t)s * slot_floats;
-        const float *src = (FUSED && row < 0 ? a.Dvec + (size_t)(-row - 1) * a.De : a.Qtab + (size_t)row * a.De) + ubeg * V;
-        mbar_expect_tx(bar, segbytes * H);
-        bulk_g2s(dst, src, segbytes, bar);
-        if constexpr (CPLX) bulk_g2s(dst + HSTR, src + a.d, segbytes, bar);
-      }
+      const float *src = (FUSED && row < 0 ? a.Dvec + (size_t)(uint32_t)(-row - 1) * (uint32_t)a.De
+                                           : a.Qtab + (size_t)(uint32_t)row * (uint32_t)a.De) + ubeg * V;
+      const uint32_t dst = slots_s + (uint32_t)(s * slot_floats) * 4u;
+      bulk_g2s_warp<H, false>(bars_s + 8u * s, dst, src, dst + HSTR * 4u, src + a.d, segbytes);
     };
     for (int k = 0; k < D; ++k)
       if (beg + k < end) issue(k, beg + k);
@@ -803,12 +808,14 @@ __global__ void __launch_bounds__(entity_warps(S, FUSED) * 32, 1) entity_kernel(
     const int nact = (ucnt + 31) >> 5;                    // chunks holding at least one unit: the same for every lane
     int s = 0;
     for (int i = beg; i < end; ++i) {
-      mbar_wait(bars + s, (par >> s) & 1u);
+      // (dL/ds, perm entry) of pair i from the window registers; FUSED: perm entry < 0 = direct gradient row
+      const bool cur = i >= pbase;
+      const int wl = i - pbase + (cur ? 0 : 32);
+      const float g = __shfl_sync(0xffffffffu, cur ? pg : pg0, wl);
+      const int row = FUSED ? __shfl_sync(0xffffffffu, cur ? prow : prow0, wl) : 0;
+      mbar_wait(bars_s + 8u * s, (par >> s) & 1u);
       par ^= 1u << s;
       const float *ql = slots + (size_t)s * slot_floats + lane * V;
-      const float2 mt = meta[s];
-      const float g = mt.x;
-      const int row = __float_as_int(mt.y);
       const float go = dsum_of<MODEL>(g, modulus);
       float vsum = 0.f;
       if (FUSED && row < 0) {
